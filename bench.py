@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (one rank per GPU; torchrun for N > 1)
   python bench.py --impl reference ...                     the reference's own CPU implementation (oracle/_ref) beside it
+  python bench.py ... --dump-outputs DIR                   also writes what the last timed step returned, as DIR/<name>.npy
 
 A "step" is ONE full VAMP iteration (Gaussian-mixture denoiser + EM prior update + LMMSE conjugate-gradient solve +
 Onsager solve + noise-precision update + metrics) on the synthetic i.i.d. design of the headline configuration, markers
@@ -39,6 +40,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (it may be read-only)
 sys.path.insert(0, ROOT)
 
 METRIC = "vamp_iterations_per_s"
@@ -72,6 +74,8 @@ def parse_args():
     ap.add_argument("--no-ab", action="store_true", help="skip the short device-resident legs of the other schedules")
     ap.add_argument("--storage", default="f64", choices=["f64", "f32"],
                     help="f32 = opt-in mode that holds the matrix rounded to FP32 in HBM (arithmetic FP64); NOT the headline configuration")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed legs, write what their last step returned as DIR/<name>.npy "
+                                                          "(float64), so that two builds can be compared output for output")
     return ap.parse_args()
 
 
@@ -387,6 +391,36 @@ def parity_block(world, rank, local, new_comm_id, allsum, schedule):
 
 
 # ------------------------------------------------------------------------------------------------------------------
+# outputs of the timed path (--dump-outputs)
+# ------------------------------------------------------------------------------------------------------------------
+DUMP_MAX_VALUES = 1 << 21       # per marker vector: x1_hat, r1 and the sample's index stay under 64 MB in all
+DUMP_SAMPLE_SEED = 2027
+DUMP_NAMES = ("params", "metrics", "prior_probs", "prior_vars", "cg_iters", "nmse", "sample_index", "x1_hat", "r1")
+
+
+def dump_outputs(out_dir, last, x1, r1):
+    """Writes what the last timed step handed its caller: the scalars returned by the step of the device-resident leg (the
+    headline value), and x1_hat/sqrt(N), r1/sqrt(N) as the step of the end-to-end leg copied them to host memory (the same
+    iteration W+K of an identically initialised solver), over all markers in global order. A vector longer than
+    DUMP_MAX_VALUES is replaced by its entries at a fixed seeded sample of marker indices, written as sample_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name in DUMP_NAMES:           # a file of an earlier dump (sample_index.npy of a larger run) must not sit beside this one's
+        path = os.path.join(out_dir, name + ".npy")
+        if os.path.exists(path):
+            os.remove(path)
+    arrays = {"params": last["params"], "metrics": last["metrics"], "prior_probs": last["probs"], "prior_vars": last["vars"],
+              "cg_iters": [last["k1"], last["k2"]], "nmse": [last["nmse"]]}
+    if x1.size > DUMP_MAX_VALUES:
+        idx = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(x1.size, DUMP_MAX_VALUES, replace=False))
+        x1, r1 = x1[idx], r1[idx]
+        arrays["sample_index"] = idx
+    arrays.update(x1_hat=x1, r1=r1)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+    return sorted(arrays)
+
+
+# ------------------------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------------------------
 def main_ours(args):
@@ -537,6 +571,15 @@ def main_ours(args):
 
     ms_dev, hist_dev, prof_dev, cnt_dev = leg(e2e=False)
     ms_e2e, hist_e2e, prof_e2e, cnt_e2e = leg(e2e=True)
+    dumped = None
+    if args.dump_outputs:
+        x1_all, r1_all = x1_host.numpy().copy(), r1_host.numpy().copy()
+        if world > 1:                 # shards in rank order are the markers in global order (divide_work)
+            parts = [None] * world
+            dist.all_gather_object(parts, (x1_all, r1_all))
+            x1_all, r1_all = np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts])
+        if rank == 0:
+            dumped = dump_outputs(args.dump_outputs, hist_dev[-1], x1_all, r1_all)
     # the other schedules on the same box, same iterations (device-resident leg only): what each level of pass sharing buys
     ab = {}
     if not args.no_ab:
@@ -629,6 +672,8 @@ def main_ours(args):
                              "`value` above is the default schedule's", **ab}
     if parity is not None:
         line["parity"] = parity
+    if dumped:
+        line["dumped_outputs"] = {"dir": os.path.abspath(args.dump_outputs), "files": [n + ".npy" for n in dumped]}
     live_cg = [[h["k1"], h["k2"]] for h in hist_dev]
     sh.close()
     if not args.no_cpu_baseline and world == 1:

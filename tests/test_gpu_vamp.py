@@ -368,36 +368,55 @@ def _ref_cg_counts(log):
 
 @pytest.mark.parametrize("gpus", [1, 2])
 def test_mid_size_run_matches_the_reference_binary_on_this_box(gpus, tmp_path):
-    """The reference itself (oracle/_ref/main_meth_ref, built from /root/reference by oracle/build_ref.py; it travels to the
-    GPU box as a prebuilt binary) and bin/main_meth read the SAME files — N = 4 000, Mt = 20 000 (0.64 GB), --gam1 1e-2 — and
-    must agree to 1e-9 on x1_hat / r1 of every iteration, 1e-8 on the CSV values, exactly on the CG iteration counts and on
-    the CSV byte layout; with --gpus 2 the same through the marker-sharded path."""
-    if not os.path.isfile(REF_BIN):
-        pytest.skip("oracle/_ref/main_meth_ref is not present (built only where /root/reference exists)")
+    """bin/main_meth on mid-size files — N = 4 000, Mt = 20 000 (0.64 GB), --gam1 1e-2 — against the stored outputs of the
+    reference for the SAME files (tests/golden/midsize_gam1e-2.npz, written by tests/tools/make_midsize_golden.py; its `source`
+    says whether the reference binary or the numpy oracle produced it): 1e-9 on x1_hat / r1 of every iteration (at a seeded
+    sample of markers, and on the full-vector norms), 1e-8 on the CSV values, CG iteration counts exact, CSV byte layout
+    identical. Where the reference binary itself is present (oracle/_ref/main_meth_ref), the same run is also compared with a
+    live run of it, whole vectors. With --gpus 2 all of this goes through the marker-sharded path."""
     if capi.device_count() < gpus:
         pytest.skip(f"needs {gpus} GPUs")
-    N, M, its, seed = 4000, 20000, 4, 11
+    import hashlib
+    import re
+    g = load_golden("midsize_gam1e-2")
+    N, M, its, seed = int(g["N"]), int(g["M"]), int(g["iterations"]), int(g["probe_seed"])
     d = str(tmp_path)
-    sim.write_dataset(d, "mid", N, M, lam=0.01, h2=0.5, seed=77)
+    X, _, _ = sim.write_dataset(d, "mid", N, M, lam=float(g["lam"]), h2=float(g["h2"]), seed=int(g["data_seed"]))
+    assert hashlib.sha256(X.tobytes()).hexdigest() == g["sha256_A"], "numpy generator drifted: regenerate the fixture"
+    del X
     common = ["--meth-file", f"{d}/mid.bin", "--phen-file", f"{d}/mid.phen", "--N", N, "--Mt", M, "--out-name", "m", "--iterations", its,
-              "--true-signal-file", f"{d}/mid_ts.bin", "--stop-criteria-thr", 0, "--gam1", "1e-2"]
-    os.makedirs(tmp_path / "ref"); os.makedirs(tmp_path / "gpu")
+              "--true-signal-file", f"{d}/mid_ts.bin", "--stop-criteria-thr", 0, "--gam1", g["gam1"]]
+    os.makedirs(tmp_path / "gpu")
+    out = run_cli(common + ["--out-dir", f"{d}/gpu", "--seed", seed, "--gpus", gpus], timeout=900)
+    got_cg = [(int(a), int(b)) for a, b in re.findall(r"\[CG\] LMMSE solve: (\d+) iterations, onsager solve: (\d+)", out)]
+    assert got_cg == [tuple(int(v) for v in c) for c in g["cg_iters"]], "CG iteration counts"
+    idx = g["sample_index"]
+    for k in range(1, its + 1):
+        for key, f in (("x1", f"m_it_{k}.bin"), ("r1", f"m_r1_it_{k}.bin")):
+            a = np.fromfile(f"{d}/gpu/{f}")
+            assert a.size == M, f
+            assert rel_l2(a[idx], g[key][k - 1]) < 1e-9, f
+            assert abs(np.linalg.norm(a) - g[f"{key}_norm"][k - 1]) <= 1e-9 * g[f"{key}_norm"][k - 1], f
+    def csvs_match(want_of):
+        for kind in ("params", "metrics", "prior"):
+            got, want = open(f"{d}/gpu/m_{kind}.csv", "rb").read(), want_of(kind)
+            assert len(got) == len(want)
+            assert np.array_equal(np.frombuffer(got, dtype=np.uint8) == 0, np.frombuffer(want, dtype=np.uint8) == 0), f"{kind}.csv NUL layout"
+            if kind != "prior":
+                assert_rows_close(csv_rows(got), csv_rows(want), 1e-8, kind)
+
+    csvs_match(lambda kind: bytes(g[f"csv_{kind}"]))
+    if not os.path.isfile(REF_BIN):
+        return
+    os.makedirs(tmp_path / "ref")
     ref = subprocess.run([REF_BIN] + [str(a) for a in common + ["--out-dir", f"{d}/ref", "--verbosity", 1]], stdout=subprocess.PIPE,
                          stderr=subprocess.STDOUT, text=True, timeout=900, env=dict(os.environ, VAMPOMI_SEED=str(seed), OMP_NUM_THREADS=str(os.cpu_count() or 1)))
     assert ref.returncode == 0, ref.stdout[-2000:]
-    out = run_cli(common + ["--out-dir", f"{d}/gpu", "--seed", seed, "--gpus", gpus], timeout=900)
-    import re
-    got_cg = [(int(a), int(b)) for a, b in re.findall(r"\[CG\] LMMSE solve: (\d+) iterations, onsager solve: (\d+)", out)]
     assert got_cg == _ref_cg_counts(ref.stdout), "CG iteration counts"
     for k in range(1, its + 1):
         for f in (f"m_it_{k}.bin", f"m_r1_it_{k}.bin"):
             assert rel_l2(np.fromfile(f"{d}/gpu/{f}"), np.fromfile(f"{d}/ref/{f}")) < 1e-9, f
-    for kind in ("params", "metrics", "prior"):
-        got, want = open(f"{d}/gpu/m_{kind}.csv", "rb").read(), open(f"{d}/ref/m_{kind}.csv", "rb").read()
-        assert len(got) == len(want)
-        assert np.array_equal(np.frombuffer(got, dtype=np.uint8) == 0, np.frombuffer(want, dtype=np.uint8) == 0), f"{kind}.csv NUL layout"
-        if kind != "prior":
-            assert_rows_close(csv_rows(got), csv_rows(want), 1e-8, kind)
+    csvs_match(lambda kind: open(f"{d}/ref/m_{kind}.csv", "rb").read())
 
 
 def test_main_meth_probit_entry_point(tmp_path):

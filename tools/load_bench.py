@@ -16,7 +16,7 @@ import vampomi_b200 as vb  # noqa: E402
 ap = argparse.ArgumentParser()
 ap.add_argument("--N", type=int, default=20000)
 ap.add_argument("--M", type=int, default=50000)
-ap.add_argument("--big", action="store_true", help="few variants only (for a file of tens of GB): page cache, then cold disk after dropping the caches")
+ap.add_argument("--big", action="store_true", help="few variants only (for a file of tens of GB): page cache, then O_DIRECT reads that bypass it")
 a = ap.parse_args()
 d = tempfile.mkdtemp(prefix="vampomi_load_", dir="/tmp")
 path = os.path.join(d, "m.bin")
@@ -32,27 +32,16 @@ res = []
 sh.set_tuning("load_threads", 16)
 sh.load_file(path)                      # allocates the context's pinned ring once (16 threads x 3 slots): not part of any timing below
 last = sh.download(a.M - 64, 64)
-def drop_caches():
-    try:
-        os.sync()
-        with open("/proc/sys/vm/drop_caches", "w") as f:
-            f.write("3\n")
-        return True
-    except Exception:
-        return False
-
 
 if a.big:
-    for label, direct, threads, drop in (("page cache", 0, 8, False), ("page cache", 0, 16, False), ("cold disk, O_DIRECT", 1, 4, True),
-                                         ("cold disk, buffered", 0, 8, True)):
-        dropped = drop_caches() if drop else None
+    for label, direct, threads in (("page cache", 0, 8), ("page cache", 0, 16), ("O_DIRECT", 1, 4)):
         sh.set_tuning("load_threads", threads); sh.set_tuning("load_depth", 3); sh.set_tuning("load_direct", direct)
         sh.fill(0, 0.0)
         t = time.time()
         sh.load_file(path)
         dt = time.time() - t
         assert np.array_equal(sh.download(0, 64), ref) and np.array_equal(sh.download(a.M - 64, 64), last)
-        res.append(dict(source=label, caches_dropped=dropped, direct=direct, threads=threads, s=round(dt, 3), gbs=round(gb / dt, 2)))
+        res.append(dict(source=label, direct=direct, threads=threads, s=round(dt, 3), gbs=round(gb / dt, 2)))
     print(json.dumps(dict(file_gb=gb, results=res)))
     os.unlink(path)
     os.rmdir(d)
