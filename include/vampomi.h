@@ -134,6 +134,13 @@ int vampomi_load_file(vampomi_ctx* ctx, const char* path);
 /* Synthetic i.i.d. N(0,1) block generated on the device from a counter hash of (seed, global marker, sample):
  * identical for any sharding (the model of simulation/data_sim.py:35). */
 int vampomi_generate_iid(vampomi_ctx* ctx, unsigned long long seed);
+/* Missing values (opt-in; the reference has no such step): every NaN entry of a column of this shard's block, whatever its
+ * sign or payload, is replaced in HBM by the mean of that column's non-NaN entries (0 for a column without any), so the
+ * run that follows is the run on the imputed matrix. +-Inf is not missing. In FP32 storage the mean is rounded to FP32.
+ * Columns without NaN are not written. Call after load_file / upload_columns / generate_iid and before compute_stats (it
+ * invalidates the statistics). No communication: a column lives in one shard. counts, for this shard: [0] entries replaced,
+ * [1] columns with at least one NaN, [2] columns without an observed value. */
+int vampomi_impute_missing(vampomi_ctx* ctx, long long counts[3]);
 
 /* ---- marker statistics: data::compute_markers_statistics, src/data.cpp:233-283 ----------------------------- */
 int vampomi_compute_stats(vampomi_ctx* ctx, double alpha_scale);

@@ -64,6 +64,7 @@ _SIGNATURES = {
     "vampomi_download_columns": (C.c_int, [C.c_void_p, C.c_longlong, C.c_longlong, c_double_p]),
     "vampomi_load_file": (C.c_int, [C.c_void_p, C.c_char_p]),
     "vampomi_generate_iid": (C.c_int, [C.c_void_p, C.c_ulonglong]),
+    "vampomi_impute_missing": (C.c_int, [C.c_void_p, c_ll_p]),
     "vampomi_compute_stats": (C.c_int, [C.c_void_p, C.c_double]),
     "vampomi_get_stats": (C.c_int, [C.c_void_p, c_double_p, c_double_p]),
     "vampomi_atx": (C.c_int, [C.c_void_p, c_double_p, c_double_p]),
@@ -261,6 +262,13 @@ class Shard:
 
     def generate_iid(self, seed):
         _check(self.lib.vampomi_generate_iid(self.h, seed), "generate_iid")
+
+    def impute_missing(self):
+        """Replaces every NaN of a column of this shard's block by the mean of the column's other entries (0 if it has none), in
+        HBM, before compute_stats(). Returns (entries replaced, columns with a NaN, columns without an observed value)."""
+        c = (C.c_longlong * 3)()
+        _check(self.lib.vampomi_impute_missing(self.h, c), "impute_missing")
+        return c[0], c[1], c[2]
 
     def compute_stats(self, alpha_scale=1.0):
         _check(self.lib.vampomi_compute_stats(self.h, alpha_scale), "compute_stats")

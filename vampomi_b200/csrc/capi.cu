@@ -673,6 +673,23 @@ int vampomi_generate_iid(vampomi_ctx* c, unsigned long long seed) {
     return VAMPOMI_OK;
 }
 
+int vampomi_impute_missing(vampomi_ctx* c, long long counts[3]) {
+    VO_ARG(c && counts, "impute_missing: NULL argument");
+    VO_CUDA(cudaSetDevice(c->device));
+    c->stats_ready = false;
+    long long* part = reinterpret_cast<long long*>(c->red_partials);
+    int nblocks = 0;
+    VO_CHECK(launch_impute_missing(c, part, &nblocks));
+    VO_CHECK(ensure_stage(c, (size_t)3 * nblocks));
+    VO_CUDA(cudaMemcpyAsync(c->stage, part, (size_t)3 * nblocks * sizeof(long long), cudaMemcpyDeviceToHost, c->stream));
+    VO_CUDA(cudaStreamSynchronize(c->stream));
+    const long long* h = reinterpret_cast<const long long*>(c->stage);
+    counts[0] = counts[1] = counts[2] = 0;
+    for (int b = 0; b < nblocks; b++)
+        for (int k = 0; k < 3; k++) counts[k] += h[3 * b + k];
+    return VAMPOMI_OK;
+}
+
 int vampomi_compute_stats(vampomi_ctx* c, double alpha_scale) {
     VO_ARG(c, "compute_stats: NULL context");
     VO_CUDA(cudaSetDevice(c->device));

@@ -239,6 +239,7 @@ inline bool is_work_mvec(int id) {
 // ---- launchers (kernels_matrix.cu) ----
 int launch_generate_iid(vampomi_ctx* c, uint64_t seed);
 int launch_stats(vampomi_ctx* c, double alpha_scale);
+int launch_impute_missing(vampomi_ctx* c, long long* counts_dev, int* nblocks);      // counts_dev: [nblocks][3] per-block counts
 int launch_ax(vampomi_ctx* c, const double* x_dev, double* out_dev, const int* done_flag);     // incl. all-reduce and 1/sqrt(N)
 int launch_atx(vampomi_ctx* c, const double* p_dev, double* out_dev, const int* done_flag);
 int launch_loo_sums(vampomi_ctx* c, const double* w_dev, double* sums_dev);

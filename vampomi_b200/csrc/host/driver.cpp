@@ -112,6 +112,17 @@ int load_dataset(Rank& r, const std::string& phenfp, const std::string& methfp, 
     if (!r.agree(rc == 0)) return rc ? rc : 1;
     double te = now_s();
     if (r.root()) std::cout << "reading methylation data took " << te - ts << " seconds." << std::endl;   // :151
+    if (r.opt.missing == "mean") {                       // --missing mean: NaN -> column mean in HBM, before the statistics
+        long long counts[3] = {0, 0, 0};
+        rc = vampomi_impute_missing(r.ctx, counts) != VAMPOMI_OK ? fatal_abi(r, "imputing missing values") : 0;
+        const double ti = now_s();
+        if (rc == 0)
+            printf("INFO  : rank %d replaced %lld missing values by their marker's mean (%lld markers with missing values, %lld without an observed value).\n",
+                   r.rank, counts[0], counts[1], counts[2]);
+        if (!r.agree(rc == 0)) return rc ? rc : 1;
+        if (r.root()) std::cout << "imputing missing values took " << ti - te << " seconds." << std::endl;
+        te = now_s();
+    }
     if (vampomi_compute_stats(r.ctx, r.opt.alpha_scale) != VAMPOMI_OK) return fatal_abi(r, "marker statistics");
     if (r.root()) std::cout << "rank = " << r.rank << ": statistics took " << now_s() - te << " seconds to run." << std::endl;   // :281
     return 0;

@@ -114,6 +114,14 @@ bool Options::parse(int argc, char** argv, std::string* echo) {
                 return false;
             }
             ss << "--storage " << storage << "\n";
+        } else if (!strcmp(a, "--missing")) {
+            if (!need_value()) return false;
+            missing = argv[++i];
+            if (missing != "none" && missing != "mean") {
+                std::cout << "FATAL  : option --missing has to be none or mean! (" << missing << " was passed)" << std::endl;
+                return false;
+            }
+            ss << "--missing " << missing << "\n";
         } else if (!strcmp(a, "--schedule")) {
             if (!need_value()) return false;
             schedule = argv[++i];

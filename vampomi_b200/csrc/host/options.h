@@ -3,6 +3,7 @@
 // that the reference does not have: --seed (counter-hash seed of the Hutchinson probe / probit start) and --gpus; and two
 // that choose HOW the same numbers are computed: --storage (FP32 residency of the block, opt-in) and --schedule (which matrix
 // products share a read of the block: recycled (default) / fused / plain / reference, see vampomi_solver_config::fuse_passes).
+// --missing mean makes the run read a matrix with NaN entries as the matrix with each NaN replaced by its column's mean.
 #pragma once
 #include <string>
 #include <vector>
@@ -35,6 +36,7 @@ struct Options {
     bool probit_entry = false;          // entered through main_meth_probit: model forced to bin_class, probit `test` / `predict` run modes
     std::string schedule = "onepass";   // onepass | recycled | fused | plain | reference (vampomi_solver_config::fuse_passes / redundant_passes)
     std::string storage = "f64";     // "f32": hold the marker block rounded to FP32 in HBM (arithmetic stays FP64)
+    std::string missing = "none";    // "mean": replace every NaN of a marker column by the mean of its other entries (vampomi_impute_missing)
 
     // Parses argv. On error prints the reference's FATAL line to stdout and returns false (caller exits 1).
     // `echo` receives the "ardyh command line options" block the reference prints from rank 0.

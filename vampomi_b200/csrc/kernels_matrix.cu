@@ -8,6 +8,7 @@
 //
 //   reference            kernel here
 //   data::compute_markers_statistics (src/data.cpp:233-283)  k_stats
+//   (no counterpart: opt-in mean imputation of NaN entries)  k_impute_missing
 //   data::ATx / dot_product          (src/data.cpp:294-333)  k_atx
 //   data::Ax                         (src/data.cpp:340-373)  k_ax_partial + k_ax_reduce (+ all-reduce + k_scale_div)
 //   data::pvals_loo inner sums       (src/data.cpp:396-413)  k_loo_sums
@@ -111,6 +112,83 @@ int launch_stats(vampomi_ctx* c, double alpha_scale) {
     if (c->storage == 1) k_stats<float><<<blocks, 256, 0, c->stream>>>(c->A32, c->ld, c->N, c->M, alpha_scale, c->mave, c->msig);
     else k_stats<double><<<blocks, 256, 0, c->stream>>>(c->A, c->ld, c->N, c->M, alpha_scale, c->mave, c->msig);
     c->counters[0]++; c->counters[1]++; c->counters[2] += (long long)c->M * c->N * c->elem_bytes;
+    VO_CUDA(cudaGetLastError());
+    return VAMPOMI_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// missing values (opt-in, vampomi_impute_missing): every NaN of a column is replaced by the mean of the column's non-NaN
+// entries, 0 when it has none. Shaped like k_stats: one warp per column; pass 1 counts the NaNs and sums the observed
+// values in FP64 in a fixed order; pass 2 runs only for a column with a NaN, rereads it (L2 still holds it) and writes
+// the mean, rounded to T, into its NaN entries. Rows >= N (zero padding) and columns without NaN are never written.
+// Each column is read and written by its own warp only, and no entry is read after it is written, so the read-only
+// loads of V32 stay valid. counts[3*b + k], per block b: k = 0 entries replaced, 1 columns with a NaN, 2 columns
+// without an observed value; the caller sums them in block order.
+// ---------------------------------------------------------------------------------------------------------------
+template <typename T>
+__global__ void __launch_bounds__(256) k_impute_missing(T* __restrict__ A, size_t ld, int N, long long M,
+                                                        long long* __restrict__ counts) {
+    constexpr int VE = V32<T>::VE;
+    __shared__ long long tally[8][3];
+    const int lane = threadIdx.x & 31;
+    const long long warp = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const long long nwarps = (long long)gridDim.x * (blockDim.x >> 5);
+    const int nvec = N / VE;
+    long long replaced = 0, cols_nan = 0, cols_empty = 0;
+    for (long long j = warp; j < M; j += nwarps) {
+        T* col = A + (size_t)j * ld;
+        double s[4] = {0, 0, 0, 0};
+        int nan = 0;
+        for (int v = lane; v < nvec; v += 32) {
+            V32<T> a = V32<T>::cached(col + (size_t)VE * v);
+#pragma unroll
+            for (int e = 0; e < VE; e++) {
+                const double x = a.val(e);
+                if (isnan(x)) nan++;
+                else s[e & 3] += x;
+            }
+        }
+        for (int i = nvec * VE + lane; i < N; i += 32) {
+            const double x = (double)col[i];
+            if (isnan(x)) nan++;
+            else s[0] += x;
+        }
+        nan = __reduce_add_sync(0xffffffffu, nan);
+        if (nan == 0) continue;                                                   // warp-uniform: column left as it is
+        const double sum = warp_sum((s[0] + s[1]) + (s[2] + s[3]));
+        const int observed = N - nan;
+        const T fill = (T)(observed > 0 ? sum / (double)observed : 0.0);
+        for (int v = lane; v < nvec; v += 32) {
+            V32<T> a = V32<T>::cached(col + (size_t)VE * v);
+#pragma unroll
+            for (int e = 0; e < VE; e++)
+                if (isnan(a.val(e))) col[(size_t)VE * v + e] = fill;
+        }
+        for (int i = nvec * VE + lane; i < N; i += 32)
+            if (isnan((double)col[i])) col[i] = fill;
+        replaced += nan; cols_nan++; cols_empty += observed == 0;
+    }
+    if (lane == 0) {
+        tally[threadIdx.x >> 5][0] = replaced;
+        tally[threadIdx.x >> 5][1] = cols_nan;
+        tally[threadIdx.x >> 5][2] = cols_empty;
+    }
+    __syncthreads();
+    if (threadIdx.x < 3) {
+        long long t = 0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); w++) t += tally[w][threadIdx.x];
+        counts[3 * blockIdx.x + threadIdx.x] = t;
+    }
+}
+
+int launch_impute_missing(vampomi_ctx* c, long long* counts_dev, int* nblocks) {
+    int blocks = c->num_sms * 8;
+    if ((size_t)3 * blocks * sizeof(long long) > (size_t)RED_BLOCKS * MAX_SUMS * sizeof(double))   // counts live in red_partials
+        blocks = (int)((size_t)RED_BLOCKS * MAX_SUMS * sizeof(double) / (3 * sizeof(long long)));
+    if (c->storage == 1) k_impute_missing<float><<<blocks, 256, 0, c->stream>>>(c->A32, c->ld, c->N, c->M, counts_dev);
+    else k_impute_missing<double><<<blocks, 256, 0, c->stream>>>(c->A, c->ld, c->N, c->M, counts_dev);
+    c->counters[0]++; c->counters[1]++; c->counters[2] += (long long)c->M * c->N * c->elem_bytes;
+    *nblocks = blocks;
     VO_CUDA(cudaGetLastError());
     return VAMPOMI_OK;
 }
