@@ -201,47 +201,72 @@ def test_probe_matches_counter_hash():
     sh.close()
 
 
+def mixture(L):
+    """(probs, vars) of L components: the reference's defaults, or a spike and L - 1 slabs with geometric variances."""
+    if L is None:
+        return list(vo.DEFAULT_PROBS), list(vo.DEFAULT_VARS)
+    slabs = 0.5 ** np.arange(1, L)
+    return [0.9] + list(0.1 * slabs / slabs.sum()), [0.0] + list(np.geomspace(1e-6, 1.0, L - 1))
+
+
+# The vector kernels' grid-stride loops wrap from 296 x 256 = 75 776 elements on, so M = 75 777 and 200 003 give a thread two
+# or more markers; L = 32 (MAX_MIX) fills 63 of the 64 packed sums of k_em_sums. The marker block is never read by these kernels
+# and the oracle's mixture formulas need N only, so neither side gets a matrix of M columns.
+VECTOR_MS = (5000, 75777, 200003)
+MIXTURES = (None, 2, 32)
+
+
 @pytest.mark.parametrize("gam1", [1e-6, 0.37, 25.0, 1e12])
 def test_denoiser_matches_oracle(gam1):
-    N, M = 200, 5000
-    sh, A, y, rng = make(N, M, seed=4)
-    probs = np.array(vo.DEFAULT_PROBS)
-    vars_int = np.array(vo.DEFAULT_VARS) * N
-    r1 = rng.standard_normal(M) * 3
-    r1[:5] = [0.0, 1e-300, -40.0, 40.0, 1e3]
-    prev = rng.standard_normal(M)
-    o = vo.Vamp(vo.Data(A, y), vars=vo.DEFAULT_VARS, probs=vo.DEFAULT_PROBS)
-    for damp in (False, True):
-        sh.set(V_R1, r1)
-        sh.set(V_X1, prev)
-        s = sh.denoise(gam1, probs, vars_int, damp=damp, rho=0.3)
-        g, gd = o.g1(r1, gam1), o.g1d(r1, gam1)
-        want = 0.3 * g + 0.7 * prev if damp else g
-        # g1 = y + sigma*pkd/pk cancels against y when gam1 is tiny (|g1| ~ 1e-7 |y| at gam1 = 1e-6): the error budget
-        # is a few ulps of the INPUT magnitude, not of the output
-        err = np.linalg.norm(sh.get(V_X1) - want)
-        assert err <= 1e-12 * np.linalg.norm(want) + 2e-15 * np.linalg.norm(r1[np.abs(r1) < 100]), (err, np.linalg.norm(want))
-        assert np.array_equal(sh.get(V_X1_PREV), prev)
-        assert abs(s - gd.sum()) <= 1e-9 * max(abs(gd).sum(), 1.0)      # gd cancels to ~1e-8 per term when gam1 is tiny
-    sh.close()
+    N = 200
+    rng = np.random.default_rng(4)
+    data = vo.Data(rng.standard_normal((2, N)), rng.standard_normal(N))
+    for M in VECTOR_MS:
+        sh = capi.Shard(N, M)
+        r1 = rng.standard_normal(M) * 3
+        r1[:5] = [0.0, 1e-300, -40.0, 40.0, 1e3]
+        prev = rng.standard_normal(M)
+        for L in MIXTURES:
+            probs, vars_ = mixture(L)
+            vars_int = np.array(vars_) * N
+            o = vo.Vamp(data, vars=vars_, probs=probs)
+            for damp in (False, True):
+                sh.set(V_R1, r1)
+                sh.set(V_X1, prev)
+                s = sh.denoise(gam1, np.array(probs), vars_int, damp=damp, rho=0.3)
+                g, gd = o.g1(r1, gam1), o.g1d(r1, gam1)
+                want = 0.3 * g + 0.7 * prev if damp else g
+                # g1 = y + sigma*pkd/pk cancels against y when gam1 is tiny (|g1| ~ 1e-7 |y| at gam1 = 1e-6): the error budget
+                # is a few ulps of the INPUT magnitude, not of the output
+                err = np.linalg.norm(sh.get(V_X1) - want)
+                assert err <= 1e-12 * np.linalg.norm(want) + 2e-15 * np.linalg.norm(r1[np.abs(r1) < 100]), (M, L, damp, err, np.linalg.norm(want))
+                assert np.array_equal(sh.get(V_X1_PREV), prev), (M, L, damp)
+                assert abs(s - gd.sum()) <= 1e-9 * max(abs(gd).sum(), 1.0), (M, L, damp)   # gd cancels to ~1e-8 per term when gam1 is tiny
+        sh.close()
 
 
 def test_em_sums_match_oracle():
-    N, M = 150, 4000
-    sh, A, y, rng = make(N, M, seed=6)
-    r1 = rng.standard_normal(M) * 2
-    sh.set(V_R1, r1)
-    o = vo.Vamp(vo.Data(A, y))
-    probs, vars_int = list(o.probs), list(o.vars)
-    lam = 1 - probs[0]
-    omegas = [probs[0]] + [p / lam for p in probs[1:]]
-    s_pin, s_beta, s_gam = o.em_sums(r1, 0.8, lam, omegas, vars_int)
-    got = sh.em_sums(0.8, lam, omegas, vars_int)
-    L = len(probs)
-    assert np.allclose(got[0], s_pin, rtol=1e-12)
-    assert np.allclose(got[1:L], s_beta, rtol=1e-11, atol=1e-300)
-    assert np.allclose(got[L:], s_gam, rtol=1e-11, atol=1e-300)
-    sh.close()
+    N = 150
+    rng = np.random.default_rng(6)
+    data = vo.Data(rng.standard_normal((2, N)), rng.standard_normal(N))
+    for M in (4000,) + VECTOR_MS:
+        sh = capi.Shard(N, M)
+        r1 = rng.standard_normal(M) * 2
+        sh.set(V_R1, r1)
+        for L in MIXTURES:
+            probs, vars_ = mixture(L)
+            o = vo.Vamp(data, probs=probs, vars=vars_)
+            probs, vars_int = list(o.probs), list(o.vars)
+            lam = 1 - probs[0]
+            omegas = [probs[0]] + [p / lam for p in probs[1:]]
+            s_pin, s_beta, s_gam = o.em_sums(r1, 0.8, lam, omegas, vars_int)
+            got = sh.em_sums(0.8, lam, omegas, vars_int)
+            L = len(probs)
+            assert got.size == 2 * L - 1
+            assert np.allclose(got[0], s_pin, rtol=1e-12), (M, L)
+            assert np.allclose(got[1:L], s_beta, rtol=1e-11, atol=1e-300), (M, L)
+            assert np.allclose(got[L:], s_gam, rtol=1e-11, atol=1e-300), (M, L)
+        sh.close()
 
 
 def test_probit_z_channel_matches_oracle():

@@ -57,15 +57,18 @@ def kernel_order_sum(x, VE):
 
 def impute_ref(X, storage="f64"):
     """(imputed copy, [entries replaced, columns with a NaN, columns without an observed value]) of a marker-major block:
-    each NaN becomes the column's nanmean, 0 for a column without observed values. FP32 storage: X is the block as held
-    (rounded when uploaded) and the mean is rounded to FP32 too. The mean is summed in the kernel's order, so the
-    comparison does not depend on how much the column's sum cancels."""
+    each NaN becomes the column's nanmean (exactly the observed value when all observed values are equal), 0 for a column
+    without observed values. FP32 storage: X is the block as held (rounded when uploaded) and the mean is rounded to FP32
+    too. The mean is summed in the kernel's order, so the comparison does not depend on how much the column's sum cancels."""
     out = X.copy()
     miss = np.isnan(X)
     for j in np.nonzero(miss.any(axis=1))[0]:
         nobs = int((~miss[j]).sum())
+        obs = X[j][~miss[j]]
         m = kernel_order_sum(X[j], 8 if storage == "f32" else 4) / nobs if nobs else 0.0
-        if nobs:
+        if nobs and obs.min() == obs.max():
+            m = obs[0]                               # all observed values equal: exactly that value
+        elif nobs:
             assert not np.isfinite(m) or abs(m - np.nanmean(X[j])) <= 1e-12 * np.nanmean(np.abs(X[j]))
         out[j, miss[j]] = np.float32(m) if storage == "f32" else m
     return out, [int(miss.sum()), int(miss.any(axis=1).sum()), int(miss.all(axis=1).sum())]
@@ -84,8 +87,12 @@ def seeded_block(N, M, seed):
     X[5, 0] = np.inf                                 # +Inf is observed: the mean, and so the fill, is +Inf
     X[5, N - 1] = np.nan
     X[6, N // 2] = -np.inf                           # -Inf in a column without NaN: untouched
-    mask = rng.random((M - 8, N)) < 0.05             # column 7 has no NaN
-    X[8:][mask] = np.nan
+    X[8, :] = np.nan                                 # one observed value that does not sum exactly: 0.1 / 1 = 0.1, but the
+    X[8, N // 3] = 0.1                               # mean of a constant column must not depend on how it is summed
+    X[9, :] = 0.7                                    # all observed values equal (0.7 + 0.7 + ... can miss 0.7 * n by an ulp)
+    X[9, ::3] = np.nan
+    mask = rng.random((M - 10, N)) < 0.05            # column 7 has no NaN
+    X[10:][mask] = np.nan
     return X
 
 
@@ -116,10 +123,14 @@ def test_impute_kernel_matches_numpy(storage, N):
         finite = np.isfinite(want).all(axis=1)
         np.testing.assert_allclose(mave[finite], want[finite].mean(axis=1), rtol=1e-12, atol=1e-13)
         assert mave[1] == 0.0 and msig[1] == 1.0
+        for j, c in ((2, 1.25), (8, 0.1), (9, 0.7)):  # imputed columns that are constant: their value and msig = 1, exactly
+            c = float(np.float32(c)) if storage == "f32" else c
+            assert np.all(got[j] == c) and mave[j] == c and msig[j] == 1.0, (j, mave[j], msig[j])
+        const = (want.min(axis=1) == want.max(axis=1)) & finite
+        assert np.all(msig[const] == 1.0)
         if N > 2:
-            sd = want[finite].std(axis=1, ddof=1)
-            ok = sd > 0
-            np.testing.assert_allclose(msig[finite][ok], 1.0 / sd[ok], rtol=1e-11)
+            sd = want[finite & ~const].std(axis=1, ddof=1)
+            np.testing.assert_allclose(msig[finite & ~const], 1.0 / sd, rtol=1e-11)
 
 
 @pytest.mark.gpu

@@ -12,6 +12,8 @@
 //   data::ATx / dot_product          (src/data.cpp:294-333)  k_atx
 //   data::Ax                         (src/data.cpp:340-373)  k_ax_partial + k_ax_reduce (+ all-reduce + k_scale_div)
 //   data::pvals_loo inner sums       (src/data.cpp:396-413)  k_loo_sums
+#include <math_constants.h>
+
 #include "common.h"
 #include "rng.h"
 #include "vec32.cuh"
@@ -80,13 +82,22 @@ __global__ void __launch_bounds__(256) k_stats(const T* __restrict__ A, size_t l
     for (long long j = warp; j < M; j += nwarps) {
         const T* col = A + (size_t)j * ld;
         double s[4] = {0, 0, 0, 0};
+        double lo = CUDART_INF, hi = -CUDART_INF;
         for (int v = lane; v < nvec; v += 32) {
             V32<T> a = V32<T>::cached(col + (size_t)VE * v);
 #pragma unroll
-            for (int e = 0; e < VE; e++) s[e & 3] += a.val(e);
+            for (int e = 0; e < VE; e++) { const double x = a.val(e); s[e & 3] += x; lo = fmin(lo, x); hi = fmax(hi, x); }
         }
-        for (int i = nvec * VE + lane; i < N; i += 32) s[0] += (double)col[i];
+        for (int i = nvec * VE + lane; i < N; i += 32) { const double x = (double)col[i]; s[0] += x; lo = fmin(lo, x); hi = fmax(hi, x); }
         double mean = warp_sum((s[0] + s[1]) + (s[2] + s[3])) / (double)N;       // suma / nonas, src/data.cpp:258
+        warp_min_max(lo, hi);
+        // A constant column gets its own value as mean and msig = 1 (src/data.cpp:275-276), exactly: the sum above can miss a
+        // value such as 0.1 by an ulp, and then sumsqr ~ N ulp^2 != 0 gives msig ~ 1e16 and turns every standardised entry into
+        // +-1 instead of 0. fmin/fmax skip a NaN, but a NaN makes `mean` NaN, so such a column keeps the path below (NaN stats).
+        if (lo == hi && isfinite(lo) && !isnan(mean)) {                          // warp-uniform
+            if (lane == 0) { mave[j] = lo; msig[j] = 1.0; }
+            continue;
+        }
         s[0] = s[1] = s[2] = s[3] = 0;
         for (int v = lane; v < nvec; v += 32) {
             V32<T> a = V32<T>::cached(col + (size_t)VE * v);
@@ -118,9 +129,9 @@ int launch_stats(vampomi_ctx* c, double alpha_scale) {
 
 // ---------------------------------------------------------------------------------------------------------------
 // missing values (opt-in, vampomi_impute_missing): every NaN of a column is replaced by the mean of the column's non-NaN
-// entries, 0 when it has none. Shaped like k_stats: one warp per column; pass 1 counts the NaNs and sums the observed
-// values in FP64 in a fixed order; pass 2 runs only for a column with a NaN, rereads it (L2 still holds it) and writes
-// the mean, rounded to T, into its NaN entries. Rows >= N (zero padding) and columns without NaN are never written.
+// entries (exactly their value when they are all equal), 0 when it has none. Shaped like k_stats: one warp per column;
+// pass 1 counts the NaNs, sums the observed values in FP64 in a fixed order and takes their min and max; pass 2 runs only
+// for a column with a NaN, rereads it (L2 still holds it) and writes the mean, rounded to T, into its NaN entries. Rows >= N (zero padding) and columns without NaN are never written.
 // Each column is read and written by its own warp only, and no entry is read after it is written, so the read-only
 // loads of V32 stay valid. counts[3*b + k], per block b: k = 0 entries replaced, 1 columns with a NaN, 2 columns
 // without an observed value; the caller sums them in block order.
@@ -138,6 +149,7 @@ __global__ void __launch_bounds__(256) k_impute_missing(T* __restrict__ A, size_
     for (long long j = warp; j < M; j += nwarps) {
         T* col = A + (size_t)j * ld;
         double s[4] = {0, 0, 0, 0};
+        double lo = CUDART_INF, hi = -CUDART_INF;                                 // over the observed values (fmin/fmax skip NaN)
         int nan = 0;
         for (int v = lane; v < nvec; v += 32) {
             V32<T> a = V32<T>::cached(col + (size_t)VE * v);
@@ -146,18 +158,23 @@ __global__ void __launch_bounds__(256) k_impute_missing(T* __restrict__ A, size_
                 const double x = a.val(e);
                 if (isnan(x)) nan++;
                 else s[e & 3] += x;
+                lo = fmin(lo, x); hi = fmax(hi, x);
             }
         }
         for (int i = nvec * VE + lane; i < N; i += 32) {
             const double x = (double)col[i];
             if (isnan(x)) nan++;
             else s[0] += x;
+            lo = fmin(lo, x); hi = fmax(hi, x);
         }
         nan = __reduce_add_sync(0xffffffffu, nan);
         if (nan == 0) continue;                                                   // warp-uniform: column left as it is
         const double sum = warp_sum((s[0] + s[1]) + (s[2] + s[3]));
+        warp_min_max(lo, hi);
         const int observed = N - nan;
-        const T fill = (T)(observed > 0 ? sum / (double)observed : 0.0);
+        // observed values all equal: the fill is that value, so the imputed column is constant and k_stats gives it msig = 1
+        // (sum / observed can be an ulp off for a value such as 0.1)
+        const T fill = (T)(observed == 0 ? 0.0 : lo == hi ? lo : sum / (double)observed);
         for (int v = lane; v < nvec; v += 32) {
             V32<T> a = V32<T>::cached(col + (size_t)VE * v);
 #pragma unroll

@@ -88,6 +88,14 @@ __device__ __forceinline__ double warp_sum(double v) {
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
+// smallest and largest value over the warp (fmin/fmax: a NaN loses to any number)
+__device__ __forceinline__ void warp_min_max(double& lo, double& hi) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        lo = fmin(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+        hi = fmax(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+    }
+}
 
 
 }  // namespace vampomi
