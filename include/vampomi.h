@@ -145,6 +145,9 @@ int vampomi_impute_missing(vampomi_ctx* ctx, long long counts[3]);
 /* ---- marker statistics: data::compute_markers_statistics, src/data.cpp:233-283 ----------------------------- */
 int vampomi_compute_stats(vampomi_ctx* ctx, double alpha_scale);
 int vampomi_get_stats(vampomi_ctx* ctx, double* mave_M, double* msig_M);
+/* const_M[j] = 1 if compute_stats found column j constant (no NaN, min == max, finite: mave = its value, msig = 1), else 0. The same
+ * decision, not a threshold on a variance; vampomi_host_loo_pvals_flagged gives such a column p = 1. */
+int vampomi_constant_columns(vampomi_ctx* ctx, unsigned char* const_M);
 
 /* ---- operators with host buffers: data::ATx (src/data.cpp:315-333) and data::Ax (src/data.cpp:340-373) ------ */
 /* out_M[j] = msig[j] * sum_i (A[i,j]-mave[j]) * p[i] * (1/sqrt(N)) */

@@ -4,6 +4,7 @@ that replaces std::random_device, and the mixture-component merge."""
 import ctypes as C
 import math
 
+import mpmath
 import numpy as np
 import pytest
 from scipy import stats as spstats
@@ -69,7 +70,137 @@ def test_students_t_pvalues_match_scipy(lib):
             got = lib.vampomi_host_linear_reg1d_pvals(x.sum(), (x * x).sum(), (x * yv).sum(), yv.sum(), (yv * yv).sum(), n)
             want = vo.linear_reg1d_pvals(x.sum(), (x * x).sum(), (x * yv).sum(), yv.sum(), (yv * yv).sum(), n)
             assert got == pytest.approx(want, rel=1e-9, abs=1e-300)
-            assert got == pytest.approx(spstats.linregress(x, yv).pvalue, rel=1e-7, abs=1e-300)
+
+
+def host_t(sumx, sumsqx, sumxy, sumy, sumsqy, n):
+    """The t statistic of host/io.cpp linear_reg1d_pvals, operation by operation in FP64 (the host is built without FP
+    contraction, so these are the same roundings); None where the host returns 1 without a t."""
+    s2y = (sumsqy - sumy * sumy / n) / (n - 1)
+    s2x = (sumsqx - sumx * sumx / n) / (n - 1)
+    sxy = (sumxy - sumx * sumy / n) / (n - 1)
+    if s2x <= 0 or s2y <= 0 or s2x * s2y == 0:
+        return None
+    r = min(1.0, max(-1.0, sxy / math.sqrt(s2x * s2y)))
+    return abs(r * math.sqrt((n - 2) / (1 - r * r))) if abs(r) < 1 else math.inf
+
+
+def t_tail(t, dof):
+    """2 P(T_dof > |t|) = I_{dof/(dof+t^2)}(dof/2, 1/2), in mpmath (40 digits)."""
+    with mpmath.workdps(40):
+        t = mpmath.mpf(t)
+        return mpmath.betainc(mpmath.mpf(dof) / 2, mpmath.mpf(1) / 2, 0, dof / (dof + t * t), regularized=True)
+
+
+def test_students_t_tail_against_mpmath(lib):
+    """The host's Student-t tail (regularised incomplete beta by a continued fraction, DLMF 8.17.22, with lgamma differences) for
+    dof 2 ... 19 998 and p from ~1 down to 1e-300, relative to mpmath at the t the host itself computed. Measured on this
+    implementation: <= 1.7e-11 at dof 3 998 and <= 8e-11 at dof 19 998 (worst near p = 1, <= 5e-12 for p < 0.05); the bound is
+    1e-10. The sums are chosen so that s2x = s2y = 1 and r = sxy, i.e. t = r sqrt((n-2)/(1-r^2)) for a target t."""
+    checked = 0
+    for dof in (2, 3, 8, 30, 98, 398, 3998, 19998):
+        n = dof + 2
+        for t in (0.0, 1e-3, 0.01, 0.5, 1.0, 2.0, 3.0, 5.0, 8.0, 12.0, 20.0, 37.0, 40.0, 100.0, 1e3, 1e5, 1e10, 1e50, 1e149):
+            r = t / math.sqrt(t * t + n - 2) if t < 1e100 else 1.0 - 1e-16
+            sums = (0.0, float(n - 1), r * (n - 1), 0.0, float(n - 1), n)
+            th = host_t(*sums)
+            want = t_tail(th, dof)
+            if want < mpmath.mpf("1e-300"):
+                continue
+            got = lib.vampomi_host_linear_reg1d_pvals(*sums)
+            assert abs(got - want) <= 1e-10 * want, (dof, t, got, float(want))
+            checked += 1
+    assert checked > 120, checked
+
+
+# ---- loo p-values entry by entry ----------------------------------------------------------------------------------------------
+LOO_CONSTANTS = [0.1, 0.7, 0.9532, 1 / 3, 0.0]
+
+
+def loo_columns(N, rng):
+    cols = [rng.beta(0.3, 0.3, N) for _ in range(6)]                     # bimodal, methylation-like
+    cols += [0.9 + 0.005 * rng.standard_normal(N) for _ in range(6)]      # offset: mean 0.9, sd 0.005
+    a = np.full(N, 0.1)
+    a[-1] = np.nextafter(0.1, 1.0)                                        # one entry off by an ulp
+    cols.append(a)
+    a = np.full(N, 0.7)
+    a[N // 2] = np.nextafter(0.7, 0.0)
+    cols.append(a)
+    cols += [np.full(N, c) for c in LOO_CONSTANTS]
+    return np.array(cols)
+
+
+def loo_bounds(x, w, c, n):
+    """The exact t of the regression of y = w + c x on x (y_mark of src/data.cpp:404-405, with the FP64 c = x1 / sqrt(N) the host
+    uses), from two-pass centred long-double sums, and the bound dt on the host's t from the conditioning of the textbook
+    formulas of linear_reg1d_pvals. Each of s2x, s2y, sxy is a difference whose terms sum to T (in absolute value); computed from
+    FP64 sums of n terms (this test's inputs) and the host's few operations it is within (n + 16) u T, relative eps = that / its
+    exact value. r = sxy / sqrt(s2x s2y) is then within dr = (n + 16) u T_xy / (n - 1) / sqrt(s2x s2y) + |r| (eps_x + eps_y) / 2 +
+    4 u |r|, and t = r sqrt((n-2)/(1-r^2)), whose derivative is sqrt(n-2) (1-r^2)^-1.5, within dt = dr sqrt(n-2) / (1 - r'^2)^1.5
+    + 4 u |t| (1 + r^2)/(1 - r^2), r' = |r| + dr. Returns (|t|, dt), dt = inf where dr >= (1 - |r|)/2: there the formula cannot
+    resolve the column (the r^2/(1-r^2) and T/result factors are >= 1/u), and only a finite p in [0, 1] is required."""
+    L = np.longdouble
+    u = L(2.0 ** -53)
+    xl, wl, cl = x.astype(L), w.astype(L), L(c)
+    yl = wl + cl * xl
+    dx, dy = xl - xl.mean(), yl - yl.mean()
+    sxx_c, syy_c, sxy_c = (dx * dx).sum(), (dy * dy).sum(), (dx * dy).sum()
+    ax, aw = np.abs(xl), np.abs(wl)
+    Tx = (xl * xl).sum() + ax.sum() ** 2 / n
+    Ty = (wl * wl).sum() + 2 * abs(cl) * (ax * aw).sum() + cl * cl * (xl * xl).sum() + (aw.sum() + abs(cl) * ax.sum()) ** 2 / n
+    Txy = (ax * aw).sum() + abs(cl) * (xl * xl).sum() + ax.sum() * (aw.sum() + abs(cl) * ax.sum()) / n
+    if sxx_c <= 0 or syy_c <= 0:
+        return None, math.inf
+    k = (n + 16) * u
+    eps_x, eps_y = k * Tx / sxx_c, k * Ty / syy_c
+    r = sxy_c / np.sqrt(sxx_c * syy_c)
+    dr = k * Txy / np.sqrt(sxx_c * syy_c) + abs(r) * ((eps_x + eps_y) / 2 + 4 * u)
+    if not dr < (1 - abs(r)) / 2:
+        return None, math.inf
+    t = abs(r) * np.sqrt(L(n - 2) / (1 - r * r))
+    rp = abs(r) + dr
+    dt = dr * np.sqrt(L(n - 2)) / (1 - rp * rp) ** L(1.5) + 4 * u * t * (1 + r * r) / (1 - r * r)
+    return float(t), float(dt)
+
+
+@pytest.mark.parametrize("N", [400, 20000])
+def test_loo_pvalues_entry_by_entry_against_mpmath(lib, N):
+    """vampomi_host_loo_pvals(_flagged) against the exact p-value of each marker's regression: p must lie within
+    [p(|t| + dt), p(|t| - dt)] (loo_bounds), widened by 1e-10 relative for the Student-t tail. Inputs are the FP64 sums of
+    raw columns (bimodal, offset, one entry off by an ulp, constants 0.1, 0.7, 0.9532, 1/3, 0) with effects from none to
+    dominant. Constant columns passed as flagged get exactly 1.0; without flags, and for the nearly constant columns, p must be
+    finite and in [0, 1]: no NaN from rounding residue."""
+    rng = np.random.default_rng(N)
+    A = loo_columns(N, rng)
+    M = A.shape[0]
+    w = rng.standard_normal(N)
+    sqrtN = math.sqrt(N)
+    x1 = np.array([(0.0, 0.3, -2.0, 30.0, 1e-3, -400.0)[j % 6] for j in range(M)]) * sqrtN
+    sums = np.ascontiguousarray(np.stack([A.sum(1), (A * A).sum(1), A @ w], axis=1))
+    const = (A.min(1) == A.max(1)).astype(np.uint8)
+    assert const.sum() == len(LOO_CONSTANTS)
+    dp = lambda a: a.ctypes.data_as(C.POINTER(C.c_double))
+    flagged, plain, zeros = np.full(M, -1.0), np.full(M, -1.0), np.full(M, -1.0)
+    lib.vampomi_host_loo_pvals_flagged(dp(x1), dp(sums), w.sum(), (w * w).sum(), N, M, const.ctypes.data_as(capi.c_u8_p), dp(flagged), 0)
+    lib.vampomi_host_loo_pvals(dp(x1), dp(sums), w.sum(), (w * w).sum(), N, M, dp(plain), 0)
+    nof = np.zeros(M, dtype=np.uint8)
+    lib.vampomi_host_loo_pvals_flagged(dp(x1), dp(sums), w.sum(), (w * w).sum(), N, M, nof.ctypes.data_as(capi.c_u8_p), dp(zeros), 0)
+    assert np.array_equal(zeros, plain)
+    lib.vampomi_host_loo_pvals_flagged(dp(x1), dp(sums), w.sum(), (w * w).sum(), N, M, None, dp(zeros), 0)
+    assert np.array_equal(zeros, plain)
+    assert np.all(np.isfinite(plain) & (plain >= 0) & (plain <= 1)), plain
+    assert np.all(flagged[const == 1] == 1.0) and np.array_equal(flagged[const == 0], plain[const == 0])
+    resolved = 0
+    for j in range(M):
+        if const[j]:
+            continue
+        t, dt = loo_bounds(A[j], w, x1[j] / sqrtN, N)
+        if not math.isfinite(dt):
+            continue
+        lo = float(t_tail(t + dt, N - 2)) * (1 - 1e-10)
+        hi = min(1.0, float(t_tail(max(0.0, t - dt), N - 2)) * (1 + 1e-10))
+        assert lo <= plain[j] <= hi, (j, plain[j], lo, hi, t, dt)
+        resolved += 1
+    assert resolved >= 12, resolved                       # the bimodal and offset columns are all resolved
 
 
 def test_loo_pvalues_of_a_marker_block_are_the_same_on_any_number_of_threads(lib):

@@ -14,6 +14,7 @@ from .build import LIB_PATH
 c_double_p = C.POINTER(C.c_double)
 c_int_p = C.POINTER(C.c_int)
 c_ll_p = C.POINTER(C.c_longlong)
+c_u8_p = C.POINTER(C.c_ubyte)
 
 MAX_MIX = 32
 
@@ -67,6 +68,7 @@ _SIGNATURES = {
     "vampomi_impute_missing": (C.c_int, [C.c_void_p, c_ll_p]),
     "vampomi_compute_stats": (C.c_int, [C.c_void_p, C.c_double]),
     "vampomi_get_stats": (C.c_int, [C.c_void_p, c_double_p, c_double_p]),
+    "vampomi_constant_columns": (C.c_int, [C.c_void_p, c_u8_p]),
     "vampomi_atx": (C.c_int, [C.c_void_p, c_double_p, c_double_p]),
     "vampomi_ax": (C.c_int, [C.c_void_p, c_double_p, c_double_p]),
     "vampomi_vec_len": (C.c_int, [C.c_void_p, C.c_int, c_ll_p]),
@@ -121,6 +123,8 @@ _SIGNATURES = {
     "vampomi_host_read_phen": (C.c_longlong, [C.c_char_p, C.c_int, c_double_p, C.c_longlong]),
     "vampomi_host_linear_reg1d_pvals": (C.c_double, [C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, C.c_int]),
     "vampomi_host_loo_pvals": (None, [c_double_p, c_double_p, C.c_double, C.c_double, C.c_int, C.c_longlong, c_double_p, C.c_int]),
+    "vampomi_host_loo_pvals_flagged": (None, [c_double_p, c_double_p, C.c_double, C.c_double, C.c_int, C.c_longlong, c_u8_p,
+                                              c_double_p, C.c_int]),
     "vampomi_host_probe_sign": (C.c_double, [C.c_ulonglong, C.c_int, C.c_ulonglong]),
     "vampomi_host_probit_p1": (None, [C.c_ulonglong, C.c_int, c_double_p]),
     "vampomi_host_merge_components": (C.c_int, [c_double_p, c_double_p, C.c_int, C.c_double]),
@@ -277,6 +281,12 @@ class Shard:
         (a, pa), (b, pb) = _out(self.M), _out(self.M)
         _check(self.lib.vampomi_get_stats(self.h, pa, pb), "get_stats")
         return a, b
+
+    def constant_columns(self):
+        """Boolean per column: compute_stats found it constant (mave = its value, msig = 1)."""
+        out = np.zeros(self.M, dtype=np.uint8)
+        _check(self.lib.vampomi_constant_columns(self.h, out.ctypes.data_as(c_u8_p)), "constant_columns")
+        return out.astype(bool)
 
     def ATx(self, p):
         p, pp = _in(p, self.N)

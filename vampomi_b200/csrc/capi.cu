@@ -365,6 +365,7 @@ int vampomi_create_ex(int device, int N, long long Mt, int nranks, int rank, int
         if (c->ld != (size_t)N) VO_CUDA(cudaMemsetAsync(a_ptr, 0, a_bytes, c->stream));    // pad rows must be zero
         VO_CUDA(cudaMalloc(&c->mave, c->mpad * sizeof(double)));
         VO_CUDA(cudaMalloc(&c->msig, c->mpad * sizeof(double)));
+        VO_CUDA(cudaMalloc(&c->mconst, c->mpad));
         for (int i = 0; i < VAMPOMI_V_NUM_M; i++) {
             VO_CUDA(cudaMalloc(&c->mvec[i], c->mpad * sizeof(double)));
             VO_CUDA(cudaMemsetAsync(c->mvec[i], 0, c->mpad * sizeof(double), c->stream));
@@ -402,7 +403,7 @@ int vampomi_destroy(vampomi_ctx* c) {
     for (auto e : c->prof_free) cudaEventDestroy(e);
     xchg_teardown(c);
     if (c->comm && c->nccl) c->nccl->CommDestroy(c->comm);
-    cudaFree(c->A); cudaFree(c->A32); cudaFree(c->mave); cudaFree(c->msig);
+    cudaFree(c->A); cudaFree(c->A32); cudaFree(c->mave); cudaFree(c->msig); cudaFree(c->mconst);
     for (auto p : c->mvec) cudaFree(p);
     for (auto p : c->nvec) cudaFree(p);
     cudaFree(c->psum); cudaFree(c->atx_partial);
@@ -708,6 +709,17 @@ int vampomi_get_stats(vampomi_ctx* c, double* mave, double* msig) {
     VO_CUDA(cudaSetDevice(c->device));
     VO_CHECK(d2h_vec(c, mave, c->mave, c->M));
     VO_CHECK(d2h_vec(c, msig, c->msig, c->M));
+    return VAMPOMI_OK;
+}
+
+int vampomi_constant_columns(vampomi_ctx* c, unsigned char* const_M) {
+    VO_ARG(c && const_M, "constant_columns: NULL argument");
+    if (!c->stats_ready) { set_error("constant_columns before compute_stats"); return VAMPOMI_ERR_STATE; }
+    VO_CUDA(cudaSetDevice(c->device));
+    VO_CHECK(ensure_stage(c, (size_t)(c->M + 7) / 8));
+    VO_CUDA(cudaMemcpyAsync(c->stage, c->mconst, (size_t)c->M, cudaMemcpyDeviceToHost, c->stream));
+    VO_CUDA(cudaStreamSynchronize(c->stream));
+    memcpy(const_M, c->stage, (size_t)c->M);
     return VAMPOMI_OK;
 }
 

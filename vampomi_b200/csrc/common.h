@@ -147,6 +147,7 @@ struct vampomi_ctx {
     float* A32 = nullptr;            // same layout in FP32 (storage 1)
     double* mave = nullptr;
     double* msig = nullptr;
+    unsigned char* mconst = nullptr; // 1 = k_stats found the column constant (mave = its value, msig = 1)
     double* mvec[VAMPOMI_V_NUM_M] = {};
     double* nvec[VAMPOMI_V_NUM_N] = {};
     double* ax_partial = nullptr;    // [K][ax_chunks][ld]

@@ -439,11 +439,14 @@ int run_association(Rank& r) {                                                  
             vampomi_vec_lincomb(r.ctx, VAMPOMI_V_USER_N1, 1.0, VAMPOMI_V_Y, -1.0, VAMPOMI_V_Z1, 1.0) != VAMPOMI_OK)
             return fatal_abi(r, "loo residual");
         std::vector<double> w((size_t)N), sums((size_t)3 * r.M);
-        if (vampomi_vec_get(r.ctx, VAMPOMI_V_USER_N1, w.data()) != VAMPOMI_OK || vampomi_loo_sums(r.ctx, VAMPOMI_V_USER_N1, sums.data()) != VAMPOMI_OK)
+        std::vector<unsigned char> constant((size_t)r.M);
+        if (vampomi_vec_get(r.ctx, VAMPOMI_V_USER_N1, w.data()) != VAMPOMI_OK || vampomi_loo_sums(r.ctx, VAMPOMI_V_USER_N1, sums.data()) != VAMPOMI_OK ||
+            vampomi_constant_columns(r.ctx, constant.data()) != VAMPOMI_OK)
             return fatal_abi(r, "loo sums");
         double sw = 0, sww = 0;
         for (double v : w) { sw += v; sww += v * v; }
-        loo_pvals(x1.data(), sums.data(), sw, sww, N, r.M, pvals.data());                      // Student-t per marker, on the host's threads
+        // Student-t per marker, on the host's threads; a constant column gets p = 1 (DESIGN §4)
+        loo_pvals(x1.data(), sums.data(), sw, sww, N, r.M, pvals.data(), 0, constant.data());
         out = o.out_dir + "/" + o.out_name + "_it_" + tag + "_pval_loo.bin";
     } else {
         return 0;                                                                              // the reference silently does nothing

@@ -183,15 +183,23 @@ double linear_reg1d_pvals(double sumx, double sumsqx, double sumxy, double sumy,
     const double s2y = (sumsqy - sumy * sumy / n) / (n - 1);
     const double s2x = (sumsqx - sumx * sumx / n) / (n - 1);
     const double sxy = (sumxy - sumx * sumy / n) / (n - 1);
-    const double rxy = sxy / std::sqrt(s2x * s2y);
+    // A variance below the formula's resolution comes out as rounding residue, zero or negative: such a column (or phenotype)
+    // explains nothing, p = 1. Residue over residue can also give |r| > 1, clamped to a perfect fit. A NaN fails every
+    // comparison and stays NaN.
+    if (s2x <= 0 || s2y <= 0 || s2x * s2y == 0) return 1.0;
+    double rxy = sxy / std::sqrt(s2x * s2y);
+    if (rxy > 1.0) rxy = 1.0;
+    if (rxy < -1.0) rxy = -1.0;
     const double t = rxy * std::sqrt((n - 2) / (1 - rxy * rxy));
     return students_t_two_sided(t > 0 ? t : (0 - t), (double)(n - 2));
 }
 
-void loo_pvals(const double* x1, const double* sums, double sw, double sww, int N, long long M, double* pvals, int threads) {
+void loo_pvals(const double* x1, const double* sums, double sw, double sww, int N, long long M, double* pvals, int threads,
+               const unsigned char* constant) {
     const double sqrtN = std::sqrt((double)N);
     auto work = [&](long long j0, long long j1) {
         for (long long j = j0; j < j1; j++) {
+            if (constant != nullptr && constant[j]) { pvals[j] = 1.0; continue; }      // DESIGN §4
             // y_mark = y_mod + x * c, c = x1_hat[j]/sqrt(N) (src/data.cpp:404-405): its sums follow from those of x and y_mod
             const double c = x1[j] / sqrtN, sx = sums[3 * j], sxx = sums[3 * j + 1], sxw = sums[3 * j + 2];
             const double sumy = sw + c * sx, sumxy = sxw + c * sxx, sumsqy = sww + 2 * c * sxw + c * c * sxx;

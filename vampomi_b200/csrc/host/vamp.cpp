@@ -790,6 +790,11 @@ void vampomi_host_loo_pvals(const double* x1_M, const double* sums_3M, double su
     vampomi_host::loo_pvals(x1_M, sums_3M, sum_w, sumsq_w, N, M, pvals_M, threads);
 }
 
+void vampomi_host_loo_pvals_flagged(const double* x1_M, const double* sums_3M, double sum_w, double sumsq_w, int N, long long M,
+                                    const unsigned char* const_M, double* pvals_M, int threads) {
+    vampomi_host::loo_pvals(x1_M, sums_3M, sum_w, sumsq_w, N, M, pvals_M, threads, const_M);
+}
+
 double vampomi_host_probe_sign(unsigned long long seed, int it, unsigned long long global_marker) {
     return vampomi::probe_sign(seed, it, global_marker);
 }

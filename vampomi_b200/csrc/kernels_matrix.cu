@@ -73,7 +73,8 @@ int launch_f32_to_f64(vampomi_ctx* c, double* dst_dense, const float* src, long 
 // ---------------------------------------------------------------------------------------------------------------
 template <typename T>
 __global__ void __launch_bounds__(256) k_stats(const T* __restrict__ A, size_t ld, int N, long long M, double alpha_scale,
-                                               double* __restrict__ mave, double* __restrict__ msig) {
+                                               double* __restrict__ mave, double* __restrict__ msig,
+                                               unsigned char* __restrict__ mconst) {
     constexpr int VE = V32<T>::VE;
     const int lane = threadIdx.x & 31;
     const long long warp = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -95,7 +96,7 @@ __global__ void __launch_bounds__(256) k_stats(const T* __restrict__ A, size_t l
         // value such as 0.1 by an ulp, and then sumsqr ~ N ulp^2 != 0 gives msig ~ 1e16 and turns every standardised entry into
         // +-1 instead of 0. fmin/fmax skip a NaN, but a NaN makes `mean` NaN, so such a column keeps the path below (NaN stats).
         if (lo == hi && isfinite(lo) && !isnan(mean)) {                          // warp-uniform
-            if (lane == 0) { mave[j] = lo; msig[j] = 1.0; }
+            if (lane == 0) { mave[j] = lo; msig[j] = 1.0; mconst[j] = 1; }
             continue;
         }
         s[0] = s[1] = s[2] = s[3] = 0;
@@ -114,14 +115,15 @@ __global__ void __launch_bounds__(256) k_stats(const T* __restrict__ A, size_t l
             }
             mave[j] = mean;
             msig[j] = sig;
+            mconst[j] = 0;
         }
     }
 }
 
 int launch_stats(vampomi_ctx* c, double alpha_scale) {
     int blocks = c->num_sms * 8;
-    if (c->storage == 1) k_stats<float><<<blocks, 256, 0, c->stream>>>(c->A32, c->ld, c->N, c->M, alpha_scale, c->mave, c->msig);
-    else k_stats<double><<<blocks, 256, 0, c->stream>>>(c->A, c->ld, c->N, c->M, alpha_scale, c->mave, c->msig);
+    if (c->storage == 1) k_stats<float><<<blocks, 256, 0, c->stream>>>(c->A32, c->ld, c->N, c->M, alpha_scale, c->mave, c->msig, c->mconst);
+    else k_stats<double><<<blocks, 256, 0, c->stream>>>(c->A, c->ld, c->N, c->M, alpha_scale, c->mave, c->msig, c->mconst);
     c->counters[0]++; c->counters[1]++; c->counters[2] += (long long)c->M * c->N * c->elem_bytes;
     VO_CUDA(cudaGetLastError());
     return VAMPOMI_OK;
