@@ -406,10 +406,10 @@ def test_multi_vector_passes_match_oracle(N, M, storage):
 
 
 @pytest.mark.parametrize("N,M", SHAPES + [(9000, 77), (20000, 300), (20480, 40), (20496, 40), (33000, 31), (40960, 10)])
-def test_fused_gram_pass_matches_the_two_products(N, M):
+def test_fused_gram_pass_matches_the_two_products_at_every_cluster_size(N, M):
     """vampomi_aat_multi_dev: t = A^T q and w = A t from ONE read of the marker block (kernels_gram.cu). Both must equal what
-    the two separate products (and the oracle) give, for every kernel shape and every cluster size that holds N, for one and
-    two vectors, on ragged sizes; untouched outputs stay untouched; results are bitwise reproducible."""
+    the two separate products (and the oracle) give, for the default cluster size and every cluster size that holds N, for
+    one and two vectors, on ragged sizes; untouched outputs stay untouched; results are bitwise reproducible."""
     rng = np.random.default_rng(N * 7 + M)
     A = rng.standard_normal((M, N)) * 0.1 + 0.5
     y = rng.standard_normal(N)
@@ -422,30 +422,28 @@ def test_fused_gram_pass_matches_the_two_products(N, M):
     want_t = [d.ATx(q) for q in qs]
     want_w = [d.Ax(t) for t in want_t]
     qin, tout, wout = [V_USER_N0, V_USER_N1], [V_R1, V_R2], [V_Z1, V_Z2]
-    rows = {0: 2560, 1: 3072, 2: 2560, 3: 2560, 4: 2560, 5: 2560, 6: 2560, 7: 2560, 8: 1280, 9: 2560, 10: 2560, 11: 2560, 12: 2560, 16: 2560, 18: 2560}
+    ld = (N + 15) // 16 * 16
+    smallest = -(-ld // 2560)                                        # a CTA holds 2 560 rows of a column
     ran = 0
-    for shape in list(range(13)) + [16, 18]:
-        sh.set_tuning("gram_shape", shape)
-        for cs in (0, 1, 2, 4, 8, 16) + ((3, 5, 6, 7, 10, 13) if shape == 18 else ()):   # the default shape: any cluster size up to 16
-            ld = (N + 15) // 16 * 16
-            maxcs = 16 if shape in (8, 11, 12, 16, 18) else 8
-            if (cs and -(-ld // cs) > rows[shape]) or cs > maxcs or (cs == 0 and -(-ld // maxcs) > rows[shape]):
-                continue                                             # this cluster size cannot hold a column of N rows
-            sh.set_tuning("gram_cluster", cs)
-            for K in (1, 2):
-                for i in range(2):
-                    sh.set(qin[i], qs[i])
-                    sh.fill(tout[i], -7.0)
-                    sh.fill(wout[i], -7.0)
-                sh.aat_multi_dev(qin[:K], tout[:K], wout[:K])
-                for i in range(K):
-                    assert rel_l2(sh.get(tout[i]), want_t[i]) < 1e-12, (shape, cs, K, i)
-                    assert rel_l2(sh.get(wout[i]), want_w[i]) < 1e-12, (shape, cs, K, i)
-                for i in range(K, 2):
-                    assert np.all(sh.get(tout[i]) == -7.0) and np.all(sh.get(wout[i]) == -7.0)
-                ran += 1
-    assert ran >= (12 if N <= 20480 else 4)                          # beyond 20 480 rows only the 16-CTA clusters of shape 11 hold a column
-    sh.set_tuning("gram_shape", 18)
+    for cs in [0] + list(range(smallest, 17)):                       # 0: the default, the smallest cluster that holds N
+        sh.set_tuning("gram_cluster", cs)
+        for K in (1, 2):
+            for i in range(2):
+                sh.set(qin[i], qs[i])
+                sh.fill(tout[i], -7.0)
+                sh.fill(wout[i], -7.0)
+            sh.aat_multi_dev(qin[:K], tout[:K], wout[:K])
+            for i in range(K):
+                assert rel_l2(sh.get(tout[i]), want_t[i]) < 1e-12, (cs, K, i)
+                assert rel_l2(sh.get(wout[i]), want_w[i]) < 1e-12, (cs, K, i)
+            for i in range(K, 2):
+                assert np.all(sh.get(tout[i]) == -7.0) and np.all(sh.get(wout[i]) == -7.0)
+            ran += 1
+    assert ran == 2 * (18 - smallest) and ran >= 4
+    if smallest > 1:
+        sh.set_tuning("gram_cluster", smallest - 1)                  # too few CTAs to hold a column
+        with pytest.raises(capi.VampomiError):
+            sh.aat_multi_dev(qin, tout, wout)
     sh.set_tuning("gram_cluster", 0)
     for clusters in (1, 3, 1000):                                    # any number of column chunks, more than there are columns included
         sh.set_tuning("gram_clusters", clusters)
@@ -646,8 +644,9 @@ def test_instrumentation_and_error_paths():
     sh.profile(False)
     assert sh.time_kernel(0, 3) > 0 and sh.time_kernel(1, 3) > 0 and sh.time_kernel(2, 1) > 0 and sh.time_kernel(3, 1) > 0
     # error paths: codes and messages, never a crash
-    with pytest.raises(capi.VampomiError, match="unknown knob"):
-        sh.set_tuning("no_such_knob", 1)
+    for knob in ("no_such_knob", "gram_shape", "gram_prefetch"):    # the last two selected fused-pass variants that no longer exist
+        with pytest.raises(capi.VampomiError, match="unknown knob"):
+            sh.set_tuning(knob, 1)
     with pytest.raises(capi.VampomiError, match="must be in"):
         sh.set_tuning("ax_rv", 99)
     with pytest.raises(capi.VampomiError, match="distinct M-vectors"):

@@ -386,33 +386,17 @@ def test_onepass_cg_recurrences_reproduce_the_two_pass_iterates():
             assert np.linalg.norm(q - d.Ax(p)) < 1e-10 * np.linalg.norm(q)
 
 
-def test_default_fused_pass_shape_is_built_into_the_product_library():
-    """The default `gram_shape` (csrc/common.h) must be a case of the shape switch OUTSIDE the experiment-only block
-    (`#ifdef VAMPOMI_GRAM_EXPERIMENTS`: timing variants with wrong results), and the library must hold its kernel."""
+def test_product_library_holds_exactly_the_fused_pass_kernels():
+    """The fused pass is one kernel, k_gram_wsx<K, CS>: the library must hold its 32 instantiations (one or two systems,
+    clusters of 1 ... 16 CTAs), no other k_gram* kernel, and none of them may use local memory."""
     import os
     import re
     import subprocess
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    default = int(re.search(r"int gram_shape = (\d+);", open(os.path.join(root, "vampomi_b200", "csrc", "common.h")).read()).group(1))
-    product_cases, depth = {}, 0
-    for line in open(os.path.join(root, "vampomi_b200", "csrc", "kernels_gram.cu")):
-        if line.startswith("#ifdef VAMPOMI_GRAM_EXPERIMENTS"):
-            depth += 1
-        elif line.startswith("#endif") and depth:
-            depth -= 1
-        m = re.match(r"\s+case (\d+): return gram_launch_wsx<K, (\d+), (\d+), (\d+), CS, (\d+)(?:, (\d+), (\d+))?>", line)
-        if m and depth == 0:
-            product_cases[int(m.group(1))] = [int(x) if x else 0 for x in m.groups()[1:]]
-        m = re.match(r"\s+if \(shape == (\d+)\) \{", line)
-        if m:
-            any_cluster_shape = int(m.group(1))                     # gram_cluster(): a shape instantiated for every cluster size 1 ... 16
-        m = re.match(r"#define VAMPOMI_GRAM_CS\(n\) case n: return gram_launch_wsx<K, (\d+), (\d+), (\d+), n, (\d+), (\d+), (\d+)>", line)
-        if m and depth == 0:
-            product_cases[any_cluster_shape] = [int(x) for x in m.groups()]
-    assert default in product_cases, (default, sorted(product_cases))
-    ncw, rp, c, prod, dbg, red = product_cases[default]
-    assert dbg == 0                                                  # DBG variants leave work out or write time stamps instead of results
     lib = os.path.join(root, "vampomi_b200", "lib", "libvampomi_cuda.so")
     out = subprocess.run(["cuobjdump", "-res-usage", lib], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True).stdout
-    for k in (1, 2):
-        assert f"k_gram_wsxILi{k}ELi{ncw}ELi{rp}ELi{c}ELi8ELi{prod}ELi{dbg}ELi{red}E" in out, (k, default)
+    usage = dict(re.findall(r"Function (\S*k_gram\S*):\s*\n\s*(.*)", out))
+    names = sorted(re.search(r"k_gram\w*", f).group(0) for f in usage)
+    assert names == sorted(f"k_gram_wsxILi{k}ELi{cs}EEEvPKdmS3_S3_NS0_7GramVecEiixdPdi14CUtensorMap_st" for k in (1, 2) for cs in range(1, 17)), names
+    for f, u in usage.items():
+        assert re.search(r"\bLOCAL:0\b", u), (f, u)

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""A/B timing of the fused pass under the same thermal state: python tools/gram_ab.py [--K 2] [--reps 20] [--rounds 3] shape[:knob=v[,knob=v]] ...
+"""A/B timing of the fused pass under the same thermal state: python tools/gram_ab.py [--K 2] [--reps 20] [--rounds 3] name[:knob=v[,knob=v]] ...
 Every round times every configuration once (bursts of `reps` launches after 2 warm-up launches), so slow drifts of the SM clock
 hit all configurations alike."""
 import argparse
@@ -22,16 +22,15 @@ sh = vb.Shard(a.N, a.M)
 sh.generate_iid(1)
 sh.compute_stats()
 which = 9 if a.K == 2 else 10
-defaults = {"gram_prefetch": 4, "gram_clusters": 0, "gram_cluster": 0}
+defaults = {"gram_clusters": 0, "gram_cluster": 0}
 res = {c: [] for c in a.configs}
 for _ in range(a.rounds):
     for c in a.configs:
-        shape, _, rest = c.partition(":")
+        _, _, rest = c.partition(":")
         knobs = dict(defaults)
         for kv in filter(None, rest.split(",")):
             k, v = kv.split("=")
             knobs[k] = int(v)
-        sh.set_tuning("gram_shape", int(shape))
         for k, v in knobs.items():
             sh.set_tuning(k, v)
         sh.time_kernel(which, 2)

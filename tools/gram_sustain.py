@@ -44,7 +44,7 @@ class Clocks(threading.Thread):
 sh = vb.Shard(a.N, a.M)
 sh.generate_iid(1)
 sh.compute_stats()
-defaults = {"gram_shape": 18, "gram_clusters": 0, "gram_cluster": 0}
+defaults = {"gram_clusters": 0, "gram_cluster": 0}
 sh.time_kernel(9, a.reps)                                      # heat-up
 for rnd in range(a.rounds):
     for c in a.configs:

@@ -7,7 +7,7 @@ import re
 import subprocess
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-WANT = [("kernels_gram.o", r"k_gram_wsxILi2ELi8ELi5ELi2ELi8ELi3ELi0ELi1E"), ("kernels_gram_k1.o", r"k_gram_wsxILi1ELi8ELi5ELi2ELi8ELi3ELi0ELi1E"),
+WANT = [("kernels_gram.o", r"k_gram_wsxILi2ELi8EE"), ("kernels_gram.o", r"k_gram_wsxILi1ELi8EE"),
         ("kernels_multi.o", r"k_ax_multiIdLi3ELi1ELi4ELi0E"), ("kernels_multi.o", r"k_ax_reduce_multiILi8E")]
 KEEP = re.compile(r"^(DFMA|DADD|DMUL|LDG|STG|LDS|STS|LDL|STL|SHFL|UBLKCP|UTMALDG|USETMAXREG|SYNCS|BAR|UCGABAR|CCTL|MEMBAR|ATOM|RED|ST\.|STAS|MAPA|UMOV|ERRBAR|FENCE)")
 print("# SASS mnemonic counts of the default kernels of an iteration (cuobjdump -sass of vampomi_b200/build/*.o, sm_100a).\n"
@@ -37,6 +37,6 @@ ptx = subprocess.run(["/usr/local/cuda/bin/nvcc", "-gencode", "arch=compute_100a
                       os.path.join(ROOT, "vampomi_b200", "csrc", "kernels_gram.cu"), "-o", "/dev/null"], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True).stdout
 lines = ptx.splitlines()
 for i, l in enumerate(lines):
-    if "k_gram_wsxILi2ELi8ELi5ELi2ELi8ELi3ELi0ELi1E" in l or "k_gram_wsxILi1ELi8ELi5ELi2ELi8ELi3ELi0ELi1E" in l:
+    if "k_gram_wsxILi2ELi8EE" in l or "k_gram_wsxILi1ELi8EE" in l:
         print("ptxas -v:", l.split("function")[-1].strip())
         print("         ", lines[i + 1].strip().replace("ptxas info    : ", ""), "|", lines[i + 2].strip().replace("ptxas info    : ", ""))

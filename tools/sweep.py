@@ -22,8 +22,8 @@ ap.add_argument("--multi", type=int, default=0, help="only the multi-vector kern
                 "back-to-back reps per variant")
 ap.add_argument("--sustained", type=int, default=0, help="also time a short list of variants with this many back-to-back reps "
                 "(seconds-long, i.e. under the power cap) instead of a burst")
-ap.add_argument("--gram", type=int, default=0, help="only the fused A^T q / A A^T q pass (kernels_gram.cu) over its shapes and "
-                "cluster counts, with this many back-to-back reps per variant")
+ap.add_argument("--gram", type=int, default=0, help="only the fused A^T q / A A^T q pass (kernels_gram.cu) over its cluster "
+                "sizes and cluster counts, with this many back-to-back reps per variant")
 a = ap.parse_args()
 
 sh = vb.Shard(a.N, a.M, storage=a.storage)
@@ -50,19 +50,13 @@ if a.gram:
     t(4, "read_probe", a.gram)
     t(5, "ax_multi_K2_default", a.gram)
     t(6, "atx_multi_K2_default", a.gram)
-    for shape in list(range(13)) + [16, 18]:
-        t(9, "gram_K2", a.gram, gram_shape=shape, gram_clusters=0)
-        t(10, "gram_K1", a.gram, gram_shape=shape, gram_clusters=0)
-    for shape in (18, 16, 11, 6, 18, 16, 11, 6):
-        t(9, "gram_K2", a.gram, gram_shape=shape, gram_clusters=0)
+    t(9, "gram_K2", a.gram, gram_cluster=0, gram_clusters=0)
+    t(10, "gram_K1", a.gram, gram_cluster=0, gram_clusters=0)
     if not a.quick:
-        for shape in (0, 1):
-            for ncl in (14, 15, 30, 45, 60):
-                t(9, "gram_K2", a.gram, gram_shape=shape, gram_clusters=ncl)
-        for shape in (0, 1):
-            for cs, ncl in ((4, 0), (4, 33), (4, 66)):
-                if a.N <= cs * (3072 if shape == 1 else 2560):
-                    t(9, "gram_K2", a.gram, gram_shape=shape, gram_cluster=cs, gram_clusters=ncl)
+        for ncl in (14, 15, 30, 45, 60):
+            t(9, "gram_K2", a.gram, gram_cluster=0, gram_clusters=ncl)
+        for cs in range(-(-a.N // 2560), 17):                  # every cluster size that holds a column (2 560 rows per CTA)
+            t(9, "gram_K2", a.gram, gram_cluster=cs, gram_clusters=0)
     best = {}
     for r in results:
         if r["kernel"] not in best or r["gbs"] > best[r["kernel"]]["gbs"]:

@@ -1088,8 +1088,7 @@ int vampomi_set_tuning(vampomi_ctx* c, const char* name, int value) {
         {"multi_ax_rv", &c->tune.multi_ax_rv, 0, 2},     {"multi_ax_unroll", &c->tune.multi_ax_unroll, 0, 8},
         {"multi_atx_impl", &c->tune.multi_atx_impl, 0, 1}, {"multi_atx_cols", &c->tune.multi_atx_cols, 0, 4},
         {"multi_atx_unroll", &c->tune.multi_atx_unroll, 0, 4}, {"multi_atx_tile", &c->tune.multi_atx_tile, 0, 16384},
-        {"cg_onepass", &c->tune.cg_onepass, 0, 1},       {"gram_shape", &c->tune.gram_shape, 0, 18},         {"gram_prefetch", &c->tune.gram_prefetch, 0, 64},
-        {"gram_cluster", &c->tune.gram_cluster, 0, 16},
+        {"cg_onepass", &c->tune.cg_onepass, 0, 1},       {"gram_cluster", &c->tune.gram_cluster, 0, 16},
         {"gram_clusters", &c->tune.gram_clusters, 0, 4096}, {"gram_refresh", &c->tune.gram_refresh, 0, 100000},
     };
     for (auto& k : knobs)

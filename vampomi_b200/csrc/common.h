@@ -125,9 +125,7 @@ struct Tuning {
     int dump_stream = 0;             // asynchronous read-outs copy on 0 = the context's stream (stream-ordered), 1 = the copy stream
     int center_split = 0;            // 1 = subtract the column mean once per sum instead of once per element (LDG variants)
     int cg_onepass = 0;              // 1 = CG iterations read the marker block ONCE (fused A^T q / A A^T q pass, kernels_gram.cu) where supported
-    int gram_shape = 18;             // fused pass: kernel shape (threads, rows per thread, columns per step, steps in flight; kernels_gram.cu)
-    int gram_prefetch = 4;           // fused pass: steps ahead that one lane per CTA pulls into L2 (cp.async.bulk.prefetch), 0 = off
-    int gram_cluster = 0;            // fused pass: CTAs per cluster = row tiles of a column (0 = smallest of 1, 2, 4, 8 that holds N)
+    int gram_cluster = 0;            // fused pass: CTAs per cluster = row tiles of a column, 1 ... 16 (0 = ceil(ld / 2560), the fewest that hold N)
     int gram_clusters = 0;           // fused pass: clusters in the grid (0 = as many as are co-resident, occupancy query)
     int gram_refresh = 0;            // one-pass CG: recompute q = A p with a pass of its own every this many iterations (0 = 32)
 };
@@ -181,7 +179,7 @@ struct vampomi_ctx {
     vampomi::NcclApi* nccl = nullptr;
     vampomi::Tuning tune;
     long long counters[4] = {0, 0, 0, 0};
-    int gram_clusters[20][17][2] = {};   // co-resident clusters of k_gram per (shape, cluster size 1 ... 16, systems), 0 = not queried yet
+    int gram_clusters[17][2] = {};   // co-resident clusters of k_gram_wsx per (cluster size 1 ... 16, systems), 0 = not queried yet
     // tensor map of the marker block for the fused pass's one-copy-per-step producer (a CUtensorMap; kernels_gram.cu), with its key
     alignas(64) unsigned char gram_tmap[128] = {};
     const void* gram_tmap_A = nullptr;

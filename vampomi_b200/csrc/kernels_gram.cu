@@ -10,20 +10,48 @@
 //     w  += (a_j - mave_j) * (msig_j * t_j)                   inner loop of data::Ax, src/data.cpp:349-362
 //
 // Column j is needed twice, but only a dot product apart — so it is kept ON CHIP between the two uses instead of being read
-// from HBM again. One column is N*8 = 160 kB at N = 20 000, too much for one SM next to q and w, so a thread-block
-// CLUSTER of CS CTAs owns a column group: CTA r holds rows [r*tile, (r+1)*tile) of q (registers), of w (registers) and of
-// the C columns of the current step (registers); the partial dot products of the CS row tiles meet through distributed
-// shared memory (one st.shared::cluster per value + one cluster barrier per step), are added in rank order — every CTA gets
-// bitwise the same t_j — and the axpy runs on the registers that still hold the centred column. D steps of C columns are
-// in flight per thread, so the cluster barrier of one step overlaps the loads of the next ones.
+// from HBM again. One column is N*8 = 160 kB at N = 20 000, too much for one SM next to q and w, so a thread-block CLUSTER of
+// CS = ceil(ld / ROWS) CTAs (1 ... 16) owns a chunk of columns: CTA r holds rows [r*tile, (r+1)*tile) of q and of w in
+// registers. The chunk is walked in steps of C = 2 columns.
 //
-// Output: t (M-vector, written by cluster rank 0) and the per-chunk partials of w, which go through the same
-// k_ax_reduce_multi (fixed-order reduction + fused peer-memory all-reduce + 1/sqrt(N)) as the A x passes.
+// A CTA is three warpgroups (THREADS = 384): two of compute warps (NCW = 8) and one SERVICE warpgroup — the communication warp,
+// the producer warp and two warps that only hand their registers over. Registers are allotted at launch as if every warp needed
+// the same (168 per thread); `setmaxnreg` then moves them: the service warpgroup drops to 96, the compute warpgroups rise to 200,
+// which their 5 row pairs of q, w and two steps of columns need. Eight compute warps put two on every scheduler.
+//
+// The columns arrive through a RING of R = 4 stages in shared memory. Each stage holds one step: ONE cp.async.bulk.tensor.3d
+// (SASS UTMALDG) per step brings both column pieces of the CTA's row tile (box 16 x tile/16 x C of the {16, ld/16, M} view of
+// the block; rows past the end of a column arrive as zeros), completing on the stage's mbarrier; the producer's lanes < C store
+// the step's two column means beside it. One issuing warp gets a bulk copy under way only every ~500-650 cycles, whatever its
+// size, so one copy per step — not one per column piece — and a warp of its own that refills a stage the moment every compute
+// warp has read it, whatever the exchange is doing.
+//
+// Step s, u = s % 4 (ring stage, exchange slot and barrier; the step loops are unrolled by four, so u is a compile-time offset
+// from one shared-window base register and the barrier parity is one bit flipped per trip):
+//   compute warp:        wait ringbar[u] -> LDS its row pairs, centre them, dot with q -> add the lane quadruples {l, l^8, l^16,
+//                        l^24} (two shuffle levels) -> red[u & 1], arrive on redbar[u];
+//                        wait wready[(s-1) & 3] -> read the weights -> axpy of step s - 1 on the registers that still hold its
+//                        centred columns (the axpy is DEFERRED by one step: a compute warp never waits for the cluster round
+//                        trip of the step it just dotted, only for the one before it)
+//   producer warp:       wait redbar[u] (every compute warp has read stage u) -> refill stage u with step s + 4
+//   communication warp:  wait redbar[u] -> add the NCW warp sums (fixed tree) and the three shuffle levels left -> st.async the
+//                        CTA's partial sums to every CTA of the cluster (slot u) -> wait full[u] -> add the CS ranks' partial
+//                        sums by a fixed tree -> t_j (cluster rank 0 stores it) and the weight msig_j * t_j -> wbuf[u], arrive
+//                        on wready[u], re-arm full[u] for step s + 4
+// Every partial sum travels as ONE st.async: an 8-byte store into the peer's shared memory that also completes 8 bytes on the
+// peer's mbarrier, so data and arrival are one message and nothing in the loop is a cluster-wide barrier. Four slots make reuse
+// safe: a CTA can only send step s + 4 after it has received step s + 3 from everybody, which every peer sends after it has
+// consumed step s. red[] has two slots: a compute warp overwrites the slot of step s (at step s + 2) only after it has waited
+// for the weights of step s, which the communication warp publishes after reading the slot. Every CTA adds the same values in
+// the same order, so all CTAs of a cluster compute bitwise the same t_j.
+//
+// Output: t (M-vector, written by cluster rank 0) and the per-chunk partials of w, which go through the same k_ax_reduce_multi
+// (fixed-order reduction + fused peer-memory all-reduce + 1/sqrt(N)) as the A x passes.
 // Algorithmic bytes per launch: N*M_local*8, for t AND w, for up to two systems.
+// How this layout was reached, and the variants it replaced, with their measurements: DESIGN.md §3b.
 #include <cuda.h>                                               // CUtensorMap (type only: the encoder is fetched through cudaGetDriverEntryPoint)
 
 #include "common.h"
-#include "vec32.cuh"
 
 namespace vampomi {
 
@@ -35,12 +63,21 @@ struct GramVec {
     const int* done[2];                // "skip me" flags (nullptr = always active)
 };
 
-// Position (in doubles) of the h-th pair of the four values of 32-byte vector v of a row tile: the 32 lanes of a warp read
-// 32 consecutive vectors, so pair h of lane l sits at ((h*32 + l)*2) inside the block — consecutive lanes, consecutive
-// 16-byte words: conflict-free LDS.128 (the natural layout would put lanes 32 bytes apart).
-__device__ __forceinline__ int qs_pos(int v, int h) { return (v >> 5) * 128 + ((h << 5) + (v & 31)) * 2; }
+// layout of a CTA, shared by the kernel and its launcher
+constexpr int GRAM_NCW = 8;                                      // compute warps: two warpgroups
+constexpr int GRAM_RP = 5;                                       // 16-byte row pairs per compute thread
+constexpr int GRAM_C = 2;                                        // columns per step
+constexpr int GRAM_R = 4;                                        // ring stages
+constexpr int GRAM_THREADS = (GRAM_NCW + 4) * 32;                // + the service warpgroup: 384
+constexpr int GRAM_ROWS = GRAM_NCW * 32 * GRAM_RP * 2;           // rows per CTA: 2 560
 
+// Shared-memory operations on 32-bit shared-window addresses: inside a cluster launch the compiler re-derives the window base of
+// every __shared__ object from SR_CgaCtaId at each use (S2R + LEA per access), so the kernel computes its addresses once.
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ uint32_t opaque_u32(uint32_t x) {       // keeps the compiler from re-deriving such an address at every use
+    asm volatile("" : "+r"(x));
+    return x;
+}
 // address of the same shared-memory location in CTA `rank` of this cluster
 __device__ __forceinline__ uint32_t mapa_u32(uint32_t saddr, uint32_t rank) {
     uint32_t r;
@@ -52,26 +89,43 @@ __device__ __forceinline__ void st_async_f64(uint32_t raddr, double v, uint32_t 
     asm volatile("st.async.shared::cluster.mbarrier::complete_tx::bytes.b64 [%0], %1, [%2];"
                  ::"r"(raddr), "l"(__double_as_longlong(v)), "r"(rbar) : "memory");
 }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-    uint32_t ok = 0, spins = 0;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-        if (!ok && ++spins > (1u << 28)) __trap();              // a protocol bug must fault, not hang the GPU
-    } while (!ok);
-}
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
-__device__ __forceinline__ void prefetch_l2_bulk(const void* p, uint32_t bytes) {
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
+__device__ __forceinline__ void mbar_init_u(uint32_t bar, uint32_t count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_expect_tx_u(uint32_t bar, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive_cta_u(uint32_t bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+__device__ __forceinline__ bool mbar_try_cta_u(uint32_t bar, uint32_t parity) {
+    uint32_t ok;
+    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
+                 : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
+    return ok != 0;
+}
+// one try_wait and one branch on the fast path; the spin counter only exists on the slow path
+__device__ __forceinline__ void mbar_spin_cta_u(uint32_t bar, uint32_t parity) {
+    if (mbar_try_cta_u(bar, parity)) return;
+    uint32_t spins = 0;
+    while (!mbar_try_cta_u(bar, parity))
+        if (++spins > (1u << 28)) __trap();                      // a protocol bug must fault, not hang the GPU
+}
+__device__ __forceinline__ double lds_f64(uint32_t addr) {
+    double v;
+    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(addr));
+    return v;
+}
+__device__ __forceinline__ double2 lds_f64x2(uint32_t addr) {
+    double2 v;
+    asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(addr));
+    return v;
+}
+__device__ __forceinline__ void sts_f64(uint32_t addr, double v) {
+    asm volatile("st.shared.f64 [%0], %1;" ::"r"(addr), "d"(v) : "memory");
 }
 
 // Pairwise (tree) sum of N values held in registers: depth log2(N) instead of N - 1 dependent additions — what the
@@ -89,854 +143,9 @@ __device__ __forceinline__ double tree_sum(const double (&v)[N]) {
     }
 }
 
-// Sums NV (1, 2, 4 or 8) values over the 32 lanes of a warp with 5 exchange levels in total: at each of the first log2(NV)
-// levels a lane hands half of its values to its partner and keeps the sums of the other half, so lane v * (32/NV) (and the
-// 32/NV - 1 lanes after it) ends up with the warp total of value v.
-template <int NV>
-__device__ __forceinline__ double warp_sum_multi(const double (&v)[NV], int lane) {
-    static_assert(NV == 1 || NV == 2 || NV == 4 || NV == 8, "1, 2, 4 or 8 values");
-    double t;
-    if constexpr (NV == 8) {
-        const bool up16 = (lane & 16) != 0, up8 = (lane & 8) != 0, up4 = (lane & 4) != 0;
-        double a[4];
-#pragma unroll
-        for (int i = 0; i < 4; i++) a[i] = (up16 ? v[i + 4] : v[i]) + __shfl_xor_sync(0xffffffffu, up16 ? v[i] : v[i + 4], 16);
-        const double b0 = (up8 ? a[2] : a[0]) + __shfl_xor_sync(0xffffffffu, up8 ? a[0] : a[2], 8);
-        const double b1 = (up8 ? a[3] : a[1]) + __shfl_xor_sync(0xffffffffu, up8 ? a[1] : a[3], 8);
-        t = (up4 ? b1 : b0) + __shfl_xor_sync(0xffffffffu, up4 ? b0 : b1, 4);
-    } else if constexpr (NV == 4) {
-        const bool up16 = (lane & 16) != 0, up8 = (lane & 8) != 0;
-        const double a0 = (up16 ? v[2] : v[0]) + __shfl_xor_sync(0xffffffffu, up16 ? v[0] : v[2], 16);
-        const double a1 = (up16 ? v[3] : v[1]) + __shfl_xor_sync(0xffffffffu, up16 ? v[1] : v[3], 16);
-        t = (up8 ? a1 : a0) + __shfl_xor_sync(0xffffffffu, up8 ? a0 : a1, 8);
-        t += __shfl_xor_sync(0xffffffffu, t, 4);
-    } else if constexpr (NV == 2) {
-        const bool up16 = (lane & 16) != 0;
-        t = (up16 ? v[1] : v[0]) + __shfl_xor_sync(0xffffffffu, up16 ? v[0] : v[1], 16);
-        t += __shfl_xor_sync(0xffffffffu, t, 8);
-        t += __shfl_xor_sync(0xffffffffu, t, 4);
-    } else {
-        t = v[0] + __shfl_xor_sync(0xffffffffu, v[0], 16);
-        t += __shfl_xor_sync(0xffffffffu, t, 8);
-        t += __shfl_xor_sync(0xffffffffu, t, 4);
-    }
-    t += __shfl_xor_sync(0xffffffffu, t, 2);
-    t += __shfl_xor_sync(0xffffffffu, t, 1);
-    return t;
-}
-
-// TPB threads, RV 32-byte vectors of a column per thread (TPB*RV*4 rows per CTA), C columns per step, D register buffers of
-// one step each, CS CTAs per cluster (row tiles of a column), QS: q held in shared memory (1) or in registers (0).
-// Register budget: 8 warps -> 255 per thread, 10 or 12 warps -> 168 (three warps share a 16 K-register scheduler partition).
-//
-// Step s of a cluster = C columns. The dot products of a step need all CS row tiles, i.e. a round trip through the cluster;
-// a step-by-step barrier would serialise that latency (~1.5 us) with the loads (0.7 us per step at HBM speed). So the
-// exchange is asynchronous and the axpy of a step is deferred by one step:
-//     iteration s:   dot(s) -> warp/CTA reduce -> st.async of the CK partial sums to every CTA of the cluster (slot s % 4)
-//                    wait for the partial sums of step s-1 (sent one iteration ago: normally already there) -> t_j
-//                    axpy(s-1) on the registers that still hold its centred columns -> reload that buffer with step s-1+D
-// Every partial sum travels as ONE st.async: an 8-byte store into the peer's shared memory that also completes 8 bytes on
-// the peer's mbarrier, so data and arrival are one message and nothing in the loop is a cluster-wide barrier. Four slots
-// make reuse safe: a CTA can only send step s+4 after it has received step s+3 from everybody, which every peer sends
-// after it has consumed step s. One lane per CTA pulls the column pieces `pf` steps ahead into L2 (cp.async.bulk.prefetch),
-// so the register loads of the D-2 steps in flight see L2 latency instead of HBM latency.
-template <int K, int TPB, int RV, int C, int D, int CS, int QS>
-__global__ void __launch_bounds__(TPB, 1) k_gram(const double* __restrict__ A, size_t ld, const double* __restrict__ mave,
-                                                 const double* __restrict__ msig, GramVec gv, int tile_rows, int cols_per_chunk,
-                                                 long long M, double scale, double* __restrict__ partial, int nchunks, int pf) {
-    constexpr int VE = 4, CK = C * K, NW = TPB / 32, QSTRIDE = TPB * RV * VE;
-    static_assert(CS * CK <= 32, "one warp sends the partial sums of a step");
-    static_assert(D >= 2, "the axpy of a step is deferred by one step");
-    extern __shared__ __align__(32) double qs[];                 // [K][QSTRIDE], swizzled (qs_pos); unused when QS == 0
-    __shared__ double red[2][NW][CK];
-    __shared__ __align__(16) double xbuf[4][CS][CK];
-    __shared__ __align__(8) uint64_t full[4];
-    bool active[K];
-    bool any = false;
-#pragma unroll
-    for (int k = 0; k < K; k++) { active[k] = gv.done[k] == nullptr || *gv.done[k] == 0; any |= active[k]; }
-    if (!any) return;                                            // identical decision in every CTA of the cluster
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    uint32_t crank;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(crank));
-    if (tid == 0) {
-#pragma unroll
-        for (int i = 0; i < 4; i++) { mbar_init(&full[i], 1); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-#pragma unroll
-        for (int i = 0; i < 4; i++) mbar_expect_tx(&full[i], CS * CK * 8);
-    }
-    const size_t rbase = (size_t)crank * tile_rows;
-    const long long c0 = (long long)blockIdx.y * cols_per_chunk;
-    long long c1 = c0 + cols_per_chunk;
-    if (c1 > M) c1 = M;
-    const uint32_t piece_bytes = rbase < ld ? (uint32_t)((ld - rbase < (size_t)tile_rows ? ld - rbase : (size_t)tile_rows) * sizeof(double)) : 0u;
-
-    const double* ap[RV];
-    bool valid[RV];
-    double qr[QS ? 1 : K][QS ? 1 : RV][VE], acc[K][RV][VE];
-#pragma unroll
-    for (int rv = 0; rv < RV; rv++) {
-        const int vi = rv * TPB + tid, off = vi * VE;
-        valid[rv] = off < tile_rows && rbase + off < ld;
-        ap[rv] = A + rbase + (valid[rv] ? off : 0);
-#pragma unroll
-        for (int k = 0; k < K; k++) {
-#pragma unroll
-            for (int e = 0; e < VE; e++) acc[k][rv][e] = 0.0;
-            PV<4> pv;
-#pragma unroll
-            for (int e = 0; e < VE; e++) pv.v[e] = 0.0;
-            if (valid[rv] && active[k]) pv = PV<4>::load(gv.q[k] + rbase + off);   // pad rows of q are zero
-            if (QS) {                                                               // every thread reads back only what it wrote itself
-                *reinterpret_cast<double2*>(qs + (size_t)k * QSTRIDE + qs_pos(vi, 0)) = make_double2(pv.v[0], pv.v[1]);
-                *reinterpret_cast<double2*>(qs + (size_t)k * QSTRIDE + qs_pos(vi, 1)) = make_double2(pv.v[2], pv.v[3]);
-            } else {
-#pragma unroll
-                for (int e = 0; e < VE; e++) qr[QS ? 0 : k][QS ? 0 : rv][e] = pv.v[e];
-            }
-        }
-    }
-    const long long nsteps = c1 > c0 ? (c1 - c0 + C - 1) / C : 0;
-    V32<double> a[D][C][RV];
-
-    auto col_of = [&](long long s, int cc) { const long long j = c0 + s * C + cc; return j < c1 ? j : c1 - 1; };   // ragged last step: a valid address, weight 0
-    auto load_step = [&](const int d, long long s) {
-        if (s < nsteps) {
-#pragma unroll
-            for (int cc = 0; cc < C; cc++) {
-                const long long j = col_of(s, cc);
-#pragma unroll
-                for (int rv = 0; rv < RV; rv++)
-                    if (valid[rv]) a[d][cc][rv] = V32<double>::stream(ap[rv] + (size_t)j * ld);
-            }
-        }
-    };
-    // mave / msig of the step after the current one (loaded one step ahead: never on the critical path), of the current
-    // step, and msig of the previous one (its axpy is still to come)
-    double m_n[C], sg_n[C], sg_c[C], sg_p[C];
-#pragma unroll
-    for (int cc = 0; cc < C; cc++) {
-        const long long j = nsteps > 0 ? col_of(0, cc) : 0;
-        m_n[cc] = __ldg(mave + j); sg_n[cc] = __ldg(msig + j); sg_c[cc] = 0.0; sg_p[cc] = 0.0;
-    }
-    cluster_sync_all();                                          // every CTA's mbarriers are armed before anybody sends
-
-    auto dot_step = [&](const int d, long long s) {
-        double m[C], pd[C][K][2];
-#pragma unroll
-        for (int cc = 0; cc < C; cc++) {
-            m[cc] = m_n[cc]; sg_p[cc] = sg_c[cc]; sg_c[cc] = sg_n[cc];
-            const long long jn = col_of(s + 1 < nsteps ? s + 1 : s, cc);
-            m_n[cc] = __ldg(mave + jn); sg_n[cc] = __ldg(msig + jn);
-#pragma unroll
-            for (int k = 0; k < K; k++) pd[cc][k][0] = pd[cc][k][1] = 0.0;
-        }
-        if (pf > 0 && tid == 32 && piece_bytes != 0 && s + pf < nsteps) {
-#pragma unroll
-            for (int cc = 0; cc < C; cc++) prefetch_l2_bulk(A + rbase + (size_t)col_of(s + pf, cc) * ld, piece_bytes);
-        }
-#pragma unroll
-        for (int rv = 0; rv < RV; rv++) {
-            if (valid[rv]) {
-                double qv[K][VE];
-#pragma unroll
-                for (int k = 0; k < K; k++) {
-                    if (QS) {
-                        const double2 lo = *reinterpret_cast<const double2*>(qs + (size_t)k * QSTRIDE + qs_pos(rv * TPB + tid, 0));
-                        const double2 hi = *reinterpret_cast<const double2*>(qs + (size_t)k * QSTRIDE + qs_pos(rv * TPB + tid, 1));
-                        qv[k][0] = lo.x; qv[k][1] = lo.y; qv[k][2] = hi.x; qv[k][3] = hi.y;
-                    } else {
-#pragma unroll
-                        for (int e = 0; e < VE; e++) qv[k][e] = qr[QS ? 0 : k][QS ? 0 : rv][e];
-                    }
-                }
-#pragma unroll
-                for (int cc = 0; cc < C; cc++) {
-#pragma unroll
-                    for (int e = 0; e < VE; e++) {
-                        const double dd = a[d][cc][rv].v[e] - m[cc];           // meth[i] - mu, src/data.cpp:304 and :360
-                        a[d][cc][rv].v[e] = dd;                                 // kept centred for the deferred axpy
-#pragma unroll
-                        for (int k = 0; k < K; k++) pd[cc][k][e & 1] = fma(dd, qv[k][e], pd[cc][k][e & 1]);
-                    }
-                }
-            }
-        }
-        // partial dot products: warp (butterfly: lane v * 32/CK ends up with value v) -> CTA (fixed order) -> one message per
-        // (value, CTA of the cluster)
-        const int rb = (int)(s & 1);
-        {
-            double v[CK];
-#pragma unroll
-            for (int cc = 0; cc < C; cc++)
-#pragma unroll
-                for (int k = 0; k < K; k++) v[cc * K + k] = pd[cc][k][0] + pd[cc][k][1];
-            const double sw = warp_sum_multi<CK>(v, lane);
-            if ((lane & (32 / CK - 1)) == 0) red[rb][wid][lane / (32 / CK)] = sw;
-        }
-        __syncthreads();
-        if (tid < CS * CK) {
-            const int ck = tid % CK, dest = tid / CK, slot = (int)(s & 3);
-            double ts = red[rb][0][ck];
-#pragma unroll
-            for (int w = 1; w < NW; w++) ts += red[rb][w][ck];
-            st_async_f64(mapa_u32(smem_u32(&xbuf[slot][crank][ck]), (uint32_t)dest), ts, mapa_u32(smem_u32(&full[slot]), (uint32_t)dest));
-        }
-    };
-    auto axpy_step = [&](const int d, long long sp) {
-        const int slot = (int)(sp & 3);
-        mbar_wait_cluster(&full[slot], (uint32_t)((sp >> 2) & 1));
-        const long long j0 = c0 + sp * C;
-        // lane (r, ck) of every warp reads ONE partial sum; the CS ranks meet by an xor butterfly (the same tree on the same
-        // values in every warp of every CTA: bitwise the same t_j everywhere), lane ck then holds the total of value ck
-        double wgt[C][K];
-        {
-            const int ck = lane % CK, r = lane / CK;
-            double tot = r < CS ? xbuf[slot][r < CS ? r : 0][ck] : 0.0;
-#pragma unroll
-            for (int o = CK; o < CK * CS && o < 32; o <<= 1) tot += __shfl_xor_sync(0xffffffffu, tot, o);
-            const int cc_l = ck / K, k_l = ck % K;
-            double sgl = sg_p[0];
-#pragma unroll
-            for (int cc = 1; cc < C; cc++) sgl = cc_l == cc ? sg_p[cc] : sgl;
-            const double tj = (sgl * tot) * scale;                              // sigma_inv * dpa (:306), then * scale (:330)
-            bool act = active[0];
-#pragma unroll
-            for (int k = 1; k < K; k++) act = k_l == k ? active[k] : act;
-            const bool live = j0 + cc_l < c1 && act;
-            if (live && crank == 0 && tid < CK) (K > 1 && k_l == 1 ? gv.t[K - 1] : gv.t[0])[j0 + cc_l] = tj;
-            const double wl = live ? sgl * tj : 0.0;                            // sig_phen_i = msig * x, src/data.cpp:354
-#pragma unroll
-            for (int cc = 0; cc < C; cc++)
-#pragma unroll
-                for (int k = 0; k < K; k++) wgt[cc][k] = __shfl_sync(0xffffffffu, wl, cc * K + k);
-        }
-        if (tid == 0) mbar_expect_tx(&full[slot], CS * CK * 8);                 // re-arm the slot for step sp + 4
-#pragma unroll
-        for (int cc = 0; cc < C; cc++)
-#pragma unroll
-            for (int rv = 0; rv < RV; rv++) {
-                if (valid[rv]) {
-#pragma unroll
-                    for (int e = 0; e < VE; e++)
-#pragma unroll
-                        for (int k = 0; k < K; k++) acc[k][rv][e] = fma(a[d][cc][rv].v[e], wgt[cc][k], acc[k][rv][e]);
-                }
-            }
-    };
-
-    // the loops over d are fully unrolled, so every index into a[][][] is a compile-time constant
-#pragma unroll
-    for (int d = 0; d < D; d++) load_step(d, (long long)d);
-    for (long long s0 = 0; s0 <= nsteps; s0 += D) {
-#pragma unroll
-        for (int d = 0; d < D; d++) {
-            const long long s = s0 + d;                                         // uniform over the cluster
-            if (s < nsteps) dot_step(d, s);
-            else if (s == nsteps) {                                             // drain: only the bookkeeping of the step that is not there
-#pragma unroll
-                for (int cc = 0; cc < C; cc++) sg_p[cc] = sg_c[cc];
-            }
-            if (s >= 1 && s <= nsteps) {
-                axpy_step((d + D - 1) % D, s - 1);
-                load_step((d + D - 1) % D, s - 1 + D);
-            }
-        }
-    }
-#pragma unroll
-    for (int k = 0; k < K; k++) {
-        if (!active[k]) continue;
-        double* prow = partial + ((size_t)k * nchunks + blockIdx.y) * ld + rbase;
-#pragma unroll
-        for (int rv = 0; rv < RV; rv++)
-            if (valid[rv]) st256(prow + (rv * TPB + tid) * VE, d4{acc[k][rv][0], acc[k][rv][1], acc[k][rv][2], acc[k][rv][3]});
-    }
-    cluster_sync_all();                                          // nobody leaves while a peer may still write into its shared memory
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// The same pass with the columns staged through SHARED memory by the bulk-copy engine (cp.async.bulk global -> shared,
-// completion on an mbarrier; SASS UBLKCP): a ring of R steps of C column pieces per CTA, so the bytes in flight per SM
-// ((R-1) * C * 20 kB at N = 20 000 with 8 row tiles) no longer cost registers — the register-staged form above can keep
-// only one or two steps in flight next to q, w and the deferred step (168 registers), i.e. 40-80 kB per SM against the
-// ~100 kB that HBM latency x bandwidth asks for. Every thread owns RP 16-byte row pairs (consecutive lanes, consecutive
-// 16-byte words: conflict-free LDS.128), copies its piece of the step from the ring into registers ONCE (the ring stage is
-// free again after the block barrier of the step) and keeps it there, centred, for the deferred axpy. q and w stay in registers.
-// ---------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cta(uint64_t* bar, uint32_t parity) {
-    uint32_t ok = 0, spins = 0;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-        if (!ok && ++spins > (1u << 28)) __trap();
-    } while (!ok);
-}
-
-template <int K, int TPB, int RP, int C, int R, int CS>
-__global__ void __launch_bounds__(TPB, 1) k_gram_bulk(const double* __restrict__ A, size_t ld, const double* __restrict__ mave,
-                                                      const double* __restrict__ msig, GramVec gv, int tile_rows, int cols_per_chunk,
-                                                      long long M, double scale, double* __restrict__ partial, int nchunks) {
-    constexpr int CK = C * K, NW = TPB / 32, PIECE = TPB * RP * 2;      // doubles per column piece slot in the ring
-    static_assert(CS * CK <= 32, "one warp sends the partial sums of a step");
-    extern __shared__ __align__(128) double ring[];              // [R][C][PIECE]
-    __shared__ double red[2][NW][CK];
-    __shared__ __align__(16) double xbuf[4][CS][CK];
-    __shared__ __align__(8) uint64_t full[4];
-    __shared__ __align__(8) uint64_t ringbar[R];
-    bool active[K];
-    bool any = false;
-#pragma unroll
-    for (int k = 0; k < K; k++) { active[k] = gv.done[k] == nullptr || *gv.done[k] == 0; any |= active[k]; }
-    if (!any) return;
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    uint32_t crank;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(crank));
-    const size_t rbase = (size_t)crank * tile_rows;
-    const long long c0 = (long long)blockIdx.y * cols_per_chunk;
-    long long c1 = c0 + cols_per_chunk;
-    if (c1 > M) c1 = M;
-    const long long nsteps = c1 > c0 ? (c1 - c0 + C - 1) / C : 0;
-    const uint32_t piece_bytes = rbase < ld ? (uint32_t)((ld - rbase < (size_t)tile_rows ? ld - rbase : (size_t)tile_rows) * sizeof(double)) : 0u;
-    auto col_of = [&](long long s, int cc) { const long long j = c0 + s * C + cc; return j < c1 ? j : c1 - 1; };
-    const bool producer = tid == TPB - 32;
-    auto issue_step = [&](long long s) {                         // producer lane: the C column pieces of step s into stage s % R
-        const int st = (int)(s % R);
-        mbar_expect_tx(&ringbar[st], C * piece_bytes);
-        if (piece_bytes != 0) {
-#pragma unroll
-            for (int cc = 0; cc < C; cc++)
-                bulk_g2s(ring + ((size_t)st * C + cc) * PIECE, A + rbase + (size_t)col_of(s, cc) * ld, piece_bytes, &ringbar[st]);
-        }
-    };
-    if (tid == 0) {
-#pragma unroll
-        for (int i = 0; i < 4; i++) mbar_init(&full[i], 1);
-#pragma unroll
-        for (int i = 0; i < R; i++) mbar_init(&ringbar[i], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-#pragma unroll
-        for (int i = 0; i < 4; i++) mbar_expect_tx(&full[i], CS * CK * 8);
-    }
-    __syncthreads();
-    if (producer)
-        for (long long s = 0; s < R && s < nsteps; s++) issue_step(s);
-
-    bool valid[RP];
-    double qr[K][RP][2], acc[K][RP][2];
-#pragma unroll
-    for (int i = 0; i < RP; i++) {
-        const int off = (i * TPB + tid) * 2;
-        valid[i] = off < tile_rows && rbase + off < ld;
-#pragma unroll
-        for (int k = 0; k < K; k++) {
-            acc[k][i][0] = acc[k][i][1] = 0.0;
-            double2 qv = make_double2(0.0, 0.0);
-            if (valid[i] && active[k]) qv = *reinterpret_cast<const double2*>(gv.q[k] + rbase + off);   // pad rows of q are zero
-            qr[k][i][0] = qv.x; qr[k][i][1] = qv.y;
-        }
-    }
-    double a[2][C][RP][2];                                       // the step being dotted and the step whose axpy is pending
-    double m_n[C], sg_n[C], sg_c[C], sg_p[C];
-#pragma unroll
-    for (int cc = 0; cc < C; cc++) {
-        const long long j = nsteps > 0 ? col_of(0, cc) : 0;
-        m_n[cc] = __ldg(mave + j); sg_n[cc] = __ldg(msig + j); sg_c[cc] = 0.0; sg_p[cc] = 0.0;
-    }
-    cluster_sync_all();                                          // every CTA's mbarriers are armed before anybody sends
-
-    auto dot_step = [&](const int b, long long s) {
-        double m[C], pd[C][K][2];
-#pragma unroll
-        for (int cc = 0; cc < C; cc++) {
-            m[cc] = m_n[cc]; sg_p[cc] = sg_c[cc]; sg_c[cc] = sg_n[cc];
-            const long long jn = col_of(s + 1 < nsteps ? s + 1 : s, cc);
-            m_n[cc] = __ldg(mave + jn); sg_n[cc] = __ldg(msig + jn);
-#pragma unroll
-            for (int k = 0; k < K; k++) pd[cc][k][0] = pd[cc][k][1] = 0.0;
-        }
-        const int st = (int)(s % R);
-        mbar_wait_cta(&ringbar[st], (uint32_t)((s / R) & 1));
-        const double* stage = ring + (size_t)st * C * PIECE;
-#pragma unroll
-        for (int cc = 0; cc < C; cc++)
-#pragma unroll
-            for (int i = 0; i < RP; i++) {
-                double2 v = make_double2(m[cc], m[cc]);          // rows this thread does not own: centred value 0
-                if (valid[i]) v = *reinterpret_cast<const double2*>(stage + (size_t)cc * PIECE + (i * TPB + tid) * 2);
-                const double d0 = v.x - m[cc], d1 = v.y - m[cc];  // meth[i] - mu, src/data.cpp:304 and :360
-                a[b][cc][i][0] = d0; a[b][cc][i][1] = d1;         // kept centred for the deferred axpy
-#pragma unroll
-                for (int k = 0; k < K; k++) {
-                    pd[cc][k][0] = fma(d0, qr[k][i][0], pd[cc][k][0]);
-                    pd[cc][k][1] = fma(d1, qr[k][i][1], pd[cc][k][1]);
-                }
-            }
-        const int rb = (int)(s & 1);
-        {
-            double v[CK];
-#pragma unroll
-            for (int cc = 0; cc < C; cc++)
-#pragma unroll
-                for (int k = 0; k < K; k++) v[cc * K + k] = pd[cc][k][0] + pd[cc][k][1];
-            const double sw = warp_sum_multi<CK>(v, lane);
-            if ((lane & (32 / CK - 1)) == 0) red[rb][wid][lane / (32 / CK)] = sw;
-        }
-        __syncthreads();                                         // also: every warp has copied stage s % R into registers
-        if (producer && s + R < nsteps) issue_step(s + R);
-        if (tid < CS * CK) {
-            const int ck = tid % CK, dest = tid / CK, slot = (int)(s & 3);
-            double ts = red[rb][0][ck];
-#pragma unroll
-            for (int w = 1; w < NW; w++) ts += red[rb][w][ck];
-            st_async_f64(mapa_u32(smem_u32(&xbuf[slot][crank][ck]), (uint32_t)dest), ts, mapa_u32(smem_u32(&full[slot]), (uint32_t)dest));
-        }
-    };
-    auto axpy_step = [&](const int b, long long sp) {
-        const int slot = (int)(sp & 3);
-        mbar_wait_cluster(&full[slot], (uint32_t)((sp >> 2) & 1));
-        const long long j0 = c0 + sp * C;
-        double wgt[C][K];
-        {
-            const int ck = lane % CK, r = lane / CK;
-            double tot = r < CS ? xbuf[slot][r < CS ? r : 0][ck] : 0.0;
-#pragma unroll
-            for (int o = CK; o < CK * CS && o < 32; o <<= 1) tot += __shfl_xor_sync(0xffffffffu, tot, o);
-            const int cc_l = ck / K, k_l = ck % K;
-            double sgl = sg_p[0];
-#pragma unroll
-            for (int cc = 1; cc < C; cc++) sgl = cc_l == cc ? sg_p[cc] : sgl;
-            const double tj = (sgl * tot) * scale;                              // sigma_inv * dpa (:306), then * scale (:330)
-            bool act = active[0];
-#pragma unroll
-            for (int k = 1; k < K; k++) act = k_l == k ? active[k] : act;
-            const bool live = j0 + cc_l < c1 && act;
-            if (live && crank == 0 && tid < CK) (K > 1 && k_l == 1 ? gv.t[K - 1] : gv.t[0])[j0 + cc_l] = tj;
-            const double wl = live ? sgl * tj : 0.0;                            // sig_phen_i = msig * x, src/data.cpp:354
-#pragma unroll
-            for (int cc = 0; cc < C; cc++)
-#pragma unroll
-                for (int k = 0; k < K; k++) wgt[cc][k] = __shfl_sync(0xffffffffu, wl, cc * K + k);
-        }
-        if (tid == 0) mbar_expect_tx(&full[slot], CS * CK * 8);                 // re-arm the slot for step sp + 4
-#pragma unroll
-        for (int cc = 0; cc < C; cc++)
-#pragma unroll
-            for (int i = 0; i < RP; i++)
-#pragma unroll
-                for (int k = 0; k < K; k++) {
-                    acc[k][i][0] = fma(a[b][cc][i][0], wgt[cc][k], acc[k][i][0]);
-                    acc[k][i][1] = fma(a[b][cc][i][1], wgt[cc][k], acc[k][i][1]);
-                }
-    };
-    for (long long s0 = 0; s0 <= nsteps; s0 += 2) {
-#pragma unroll
-        for (int b = 0; b < 2; b++) {
-            const long long s = s0 + b;
-            if (s < nsteps) dot_step(b, s);
-            else if (s == nsteps) {
-#pragma unroll
-                for (int cc = 0; cc < C; cc++) sg_p[cc] = sg_c[cc];
-            }
-            if (s >= 1 && s <= nsteps) axpy_step(b ^ 1, s - 1);
-        }
-    }
-#pragma unroll
-    for (int k = 0; k < K; k++) {
-        if (!active[k]) continue;
-        double* prow = partial + ((size_t)k * nchunks + blockIdx.y) * ld + rbase;
-#pragma unroll
-        for (int i = 0; i < RP; i++)
-            if (valid[i]) *reinterpret_cast<double2*>(prow + (i * TPB + tid) * 2) = make_double2(acc[k][i][0], acc[k][i][1]);
-    }
-    cluster_sync_all();
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// Warp-specialised form of the bulk-copy pass: NCW compute warps + ONE communication warp per CTA.
-//
-// In k_gram_bulk every warp walks through the whole chain of a step — dot, warp reduction, block barrier, CTA sum, send, wait,
-// rank sum, weights, axpy — in lock-step, so the FP64 pipes idle during every exchange (measured: 1.04 us per step of 40 kB
-// against 0.69 us of HBM time). Here the chain is split:
-//   compute warp, step s:  wait ring stage -> LDS its rows -> centre, dot with q -> warp butterfly -> partial sums to red[s&1],
-//                          arrive on redbar[s&1];  wait wready[(s-1)&3] -> read the CK weights -> axpy(s-1) on the kept registers
-//   communication warp, s: wait redbar[s&1] (all compute warps have read stage s%R: lane 0 refills it with step s+R) ->
-//                          lane (dest, ck) adds the NCW warp sums in warp order and st.async's them to CTA dest (slot s&3);
-//                          wait full[s&3] -> lane (r, ck) reads one partial, xor butterfly over the ranks -> t_j, weight ->
-//                          wbuf[s&3], arrive on wready[s&3]; cluster rank 0 stores t_j
-// Compute warps never wait for the cluster round trip of the step they just dotted — only for the one before it, which the
-// communication warp has been carrying meanwhile.
-// ---------------------------------------------------------------------------------------------------------------
-// The same operations on PRECOMPUTED 32-bit shared-window addresses: inside a cluster launch the compiler re-derives the window
-// base of every __shared__ object from SR_CgaCtaId at each use (S2R + LEA per access), which the hot loop can do without.
-__device__ __forceinline__ void mbar_wait_cta_u(uint32_t bar, uint32_t parity) {
-    uint32_t ok = 0, spins = 0;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-        if (!ok && ++spins > (1u << 28)) __trap();
-    } while (!ok);
-}
-__device__ __forceinline__ void mbar_arrive_cta_u(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster_u(uint32_t bar, uint32_t parity) {
-    uint32_t ok = 0, spins = 0;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-        if (!ok && ++spins > (1u << 28)) __trap();
-    } while (!ok);
-}
-__device__ __forceinline__ void mbar_expect_tx_u(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ double lds_f64(uint32_t addr) {
-    double v;
-    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ double2 lds_f64x2(uint32_t addr) {
-    double2 v;
-    asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ void sts_f64(uint32_t addr, double v) {
-    asm volatile("st.shared.f64 [%0], %1;" ::"r"(addr), "d"(v) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cta(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-// DIRECT = 1: every compute warp sends its own partial sums to all CTAs (one st.async per lane, no block-level stage in between)
-// DEF: how many steps the axpy of a step is deferred (DEF + 1 register buffers of one step each): 1 hides one step time of the
-// cluster round trip, 2 hides two — affordable where a CTA holds few rows (RP = 2)
-// NCOMM: 1 = one communication warp sends and receives in turn; 2 = a sender warp and a receiver warp, so that the partial sums of
-// step s+1 leave while those of step s are still on their way (needed for DEF = 2 to pay)
-template <int K, int NCW, int RP, int C, int R, int CS, int DIRECT, int DEF = 1, int NCOMM = 1>
-__global__ void __launch_bounds__((NCW + NCOMM) * 32, 1) k_gram_ws(const double* __restrict__ A, size_t ld, const double* __restrict__ mave,
-                                                              const double* __restrict__ msig, GramVec gv, int tile_rows, int cols_per_chunk,
-                                                              long long M, double scale, double* __restrict__ partial, int nchunks) {
-    constexpr int CK = C * K, CT = NCW * 32, PIECE = CT * RP * 2;      // compute threads; doubles per column piece slot in the ring
-    // the communication warp handles the CS*CK (destination or rank, value) items of a step in ROUNDS rounds of 32; with CK a
-    // power of two <= 8 a lane keeps the same value index ck = lane % CK in every round and walks the ranks lane/CK + j*32/CK
-    static_assert(CK == 1 || CK == 2 || CK == 4 || CK == 8, "values per step");
-    constexpr int ROUNDS = (CS * CK + 31) / 32, RSTEP = 32 / CK;
-    extern __shared__ __align__(128) double ring[];              // [R][C][PIECE]
-    constexpr int NSRC = DIRECT ? NCW : 1;                       // partial sums per (rank, value) that arrive per step
-    static_assert(!DIRECT || CS <= 32 / CK, "the lanes that hold value ck after the butterfly send it to the CS ranks");
-    __shared__ double red[4][NCW][CK];
-    __shared__ __align__(16) double xbuf[4][CS][NSRC][CK];
-    __shared__ __align__(8) uint64_t empty[R];
-    __shared__ __align__(16) double wbuf[4][CK];
-    __shared__ __align__(8) uint64_t full[4], wready[4], redbar[4], ringbar[R];
-    static_assert(DEF == 1, "four exchange slots are only proven safe for a deferral of one step with one communication warp");
-    static_assert(NCOMM == 1, "see DEF");
-    bool active[K];
-    bool any = false;
-#pragma unroll
-    for (int k = 0; k < K; k++) { active[k] = gv.done[k] == nullptr || *gv.done[k] == 0; any |= active[k]; }
-    if (!any) return;
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    uint32_t crank;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(crank));
-    const size_t rbase = (size_t)crank * tile_rows;
-    const long long c0 = (long long)blockIdx.y * cols_per_chunk;
-    long long c1 = c0 + cols_per_chunk;
-    if (c1 > M) c1 = M;
-    // steps, stage indices and column offsets are 32-bit (a chunk has far fewer than 2^31 columns): the loop bookkeeping of the
-    // first version — 64-bit products and divisions, register moves feeding predicated loads — was 45 % of the instructions issued
-    const int ncols = c1 > c0 ? (int)(c1 - c0) : 0;
-    const int nsteps = (ncols + C - 1) / C;
-    const uint32_t piece_bytes = rbase < ld ? (uint32_t)((ld - rbase < (size_t)tile_rows ? ld - rbase : (size_t)tile_rows) * sizeof(double)) : 0u;
-    const double* const mave_c = mave + c0;                      // this chunk's statistics and columns
-    const double* const msig_c = msig + c0;
-    auto col_of = [&](int s, int cc) { const int j = s * C + cc; return j < ncols ? j : ncols - 1; };   // offset inside the chunk; ragged last step clamped
-    // rows of the ring slots that no bulk copy ever writes (the tile's tail, or all of it for a CTA without rows) are zeroed once:
-    // every compute thread can then load its row pairs unconditionally — a zero row has q = 0 and its w is never stored
-    for (int i = (int)(piece_bytes / 8) + tid; i < PIECE; i += blockDim.x)
-#pragma unroll
-        for (int sc = 0; sc < R * C; sc++) ring[(size_t)sc * PIECE + i] = 0.0;
-    if (tid == 0) {
-#pragma unroll
-        for (int i = 0; i < 4; i++) { mbar_init(&full[i], 1); mbar_init(&wready[i], 1); }
-#pragma unroll
-        for (int i = 0; i < 4; i++) mbar_init(&redbar[i], NCW);
-#pragma unroll
-        for (int i = 0; i < R; i++) { mbar_init(&ringbar[i], 1); mbar_init(&empty[i], NCW); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-#pragma unroll
-        for (int i = 0; i < 4; i++) mbar_expect_tx(&full[i], CS * NSRC * CK * 8);
-    }
-    __syncthreads();
-    cluster_sync_all();                                          // every CTA's mbarriers are armed before anybody sends
-
-    if (wid >= NCW) {
-        // ------------------------------------------- communication warp(s) -------------------------------------------
-        const bool do_send = NCOMM == 1 || wid == NCW, do_recv = NCOMM == 1 || wid == NCW + 1;
-        const double* const a_c = A + rbase + (size_t)c0 * ld;
-        auto issue_step = [&](int s) {                           // lane 0: the C column pieces of step s into stage s % R
-            const int st = s % R;
-            mbar_expect_tx(&ringbar[st], C * piece_bytes);
-            if (piece_bytes != 0) {
-#pragma unroll
-                for (int cc = 0; cc < C; cc++)
-                    bulk_g2s(ring + (st * C + cc) * PIECE, a_c + (size_t)col_of(s, cc) * ld, piece_bytes, &ringbar[st]);
-            }
-        };
-        if (lane == 0 && do_send)
-            for (int s = 0; s < R && s < nsteps; s++) issue_step(s);
-        const int ck = lane % CK, r0 = lane / CK, cc_l = ck / K, k_l = ck % K;
-        bool act = active[0];
-#pragma unroll
-        for (int k = 1; k < K; k++) act = k_l == k ? active[k] : act;
-        double* tout = K > 1 && k_l == 1 ? gv.t[K - 1] : gv.t[0];
-        double sg_next = nsteps > 0 ? __ldg(msig_c + col_of(0, cc_l)) : 0.0;
-        // everything the per-step chain addresses, as 32-bit shared-window addresses computed once: the local barriers and buffers,
-        // and — through mapa — this lane's slot in every destination CTA's receive buffer and that CTA's arrival barrier
-        const uint32_t redbar_u = smem_u32(&redbar[0]), full_u = smem_u32(&full[0]), wready_u = smem_u32(&wready[0]);
-        const uint32_t red_u = smem_u32(&red[0][0][ck]), xbuf_u = smem_u32(&xbuf[0][0][0][ck]), wbuf_u = smem_u32(&wbuf[0][ck]);
-        uint32_t rx[ROUNDS], rf[ROUNDS];                         // slot 0 of destination r0 + j*RSTEP; other slots at fixed strides
-#pragma unroll
-        for (int j = 0; j < ROUNDS; j++) {
-            const uint32_t dest = (uint32_t)(r0 + j * RSTEP < CS ? r0 + j * RSTEP : 0);
-            rx[j] = mapa_u32(smem_u32(&xbuf[0][crank][0][ck]), dest);
-            rf[j] = mapa_u32(full_u, dest);
-        }
-        constexpr uint32_t XSLOT = CS * NSRC * CK * 8, XRANK = NSRC * CK * 8;
-        for (int s = 0; s < nsteps; s++) {
-            const int rb = s & 3, slot = s & 3;
-            const double sgl = sg_next;
-            sg_next = __ldg(msig_c + col_of(s + 1 < nsteps ? s + 1 : s, cc_l));
-            if (do_send) {
-            if (DIRECT) {
-                if (lane == 0 && s + R < nsteps) {               // refill stage s % R once every compute warp has copied it into registers
-                    mbar_wait_cta(&empty[s % R], (uint32_t)((s / R) & 1));
-                    issue_step(s + R);
-                }
-            } else {
-                mbar_wait_cta_u(redbar_u + 8u * rb, (uint32_t)((s >> 2) & 1));
-                if (lane == 0 && s + R < nsteps) issue_step(s + R);  // every compute warp has copied stage s % R into registers
-                double pw[NCW];                                  // every lane: the CTA's sum of value ck over the warps (fixed tree)
-#pragma unroll
-                for (int w = 0; w < NCW; w++) pw[w] = lds_f64(red_u + (uint32_t)((rb * NCW + w) * CK * 8));
-                const double ts = tree_sum<NCW>(pw);
-#pragma unroll
-                for (int j = 0; j < ROUNDS; j++)                 // lane = (destination r0 + j*RSTEP, value ck)
-                    if (r0 + j * RSTEP < CS) st_async_f64(rx[j] + slot * XSLOT, ts, rf[j] + 8u * slot);
-            }
-            }
-            if (!do_recv) continue;
-            mbar_wait_cluster_u(full_u + 8u * slot, (uint32_t)((s >> 2) & 1));
-            // every lane reads the CS partial sums of its value ck itself and adds them by the same fixed tree: bitwise the same
-            // t_j in every CTA of the cluster, and no shuffle on the latency chain
-            double pr[CS];
-#pragma unroll
-            for (int r = 0; r < CS; r++) {
-                pr[r] = lds_f64(xbuf_u + slot * XSLOT + r * XRANK);
-#pragma unroll
-                for (int w = 1; w < NSRC; w++) pr[r] += lds_f64(xbuf_u + slot * XSLOT + r * XRANK + w * CK * 8);
-            }
-            const double tot = tree_sum<CS>(pr);
-            const int j = s * C + cc_l;
-            const double tj = (sgl * tot) * scale;                              // sigma_inv * dpa (:306), then * scale (:330)
-            const bool live = j < ncols && act;
-            if (lane < CK) {
-                if (live && crank == 0) tout[c0 + j] = tj;
-                sts_f64(wbuf_u + (uint32_t)(slot * CK * 8), live ? sgl * tj : 0.0);   // sig_phen_i = msig * x, src/data.cpp:354
-            }
-            __syncwarp();
-            if (lane == 0) {
-                mbar_arrive_cta_u(wready_u + 8u * slot);
-                mbar_expect_tx_u(full_u + 8u * slot, CS * NSRC * CK * 8);       // re-arm the slot for step s + 4
-            }
-        }
-    } else {
-        // ---------------------------------------------- compute warps ----------------------------------------------
-        bool valid[RP];
-        double qr[K][RP][2], acc[K][RP][2];
-#pragma unroll
-        for (int i = 0; i < RP; i++) {
-            const int off = (i * CT + tid) * 2;
-            valid[i] = off < tile_rows && rbase + off < ld;
-#pragma unroll
-            for (int k = 0; k < K; k++) {
-                acc[k][i][0] = acc[k][i][1] = 0.0;
-                double2 qv = make_double2(0.0, 0.0);
-                if (valid[i] && active[k]) qv = *reinterpret_cast<const double2*>(gv.q[k] + rbase + off);   // pad rows of q are zero
-                qr[k][i][0] = qv.x; qr[k][i][1] = qv.y;
-            }
-        }
-        double a[DEF + 1][C][RP][2];                             // the step being dotted and the DEF steps whose axpy is pending
-        double m_n[C];
-#pragma unroll
-        for (int cc = 0; cc < C; cc++) m_n[cc] = nsteps > 0 ? __ldg(mave_c + col_of(0, cc)) : 0.0;
-        // shared-window addresses of everything the loop touches, computed once
-        const uint32_t rows_u = smem_u32(ring) + (uint32_t)tid * 16u;            // this thread's first row pair inside a ring slot
-        const uint32_t ringbar_u = smem_u32(&ringbar[0]), redbar_u = smem_u32(&redbar[0]), wready_u = smem_u32(&wready[0]);
-        const uint32_t red_u = smem_u32(&red[0][wid][0]), wbuf_u = smem_u32(&wbuf[0][0]);
-
-        auto dot_step = [&](const int b, int s) {
-            double m[C], pd[C][K][2];
-#pragma unroll
-            for (int cc = 0; cc < C; cc++) {
-                m[cc] = m_n[cc];
-                m_n[cc] = __ldg(mave_c + col_of(s + 1 < nsteps ? s + 1 : s, cc));
-#pragma unroll
-                for (int k = 0; k < K; k++) pd[cc][k][0] = pd[cc][k][1] = 0.0;
-            }
-            const int st = s % R;
-            mbar_wait_cta_u(ringbar_u + 8u * st, (uint32_t)((s / R) & 1));
-            const uint32_t stage = rows_u + (uint32_t)(st * C * PIECE * 8);
-#pragma unroll
-            for (int cc = 0; cc < C; cc++)
-#pragma unroll
-                for (int i = 0; i < RP; i++) {
-                    const double2 v = lds_f64x2(stage + (uint32_t)((cc * PIECE + i * CT * 2) * 8));         // rows beyond the tile read zeros
-                    const double d0 = v.x - m[cc], d1 = v.y - m[cc];            // meth[i] - mu, src/data.cpp:304 and :360
-                    a[b][cc][i][0] = d0; a[b][cc][i][1] = d1;                   // kept centred for the deferred axpy
-#pragma unroll
-                    for (int k = 0; k < K; k++) {
-                        pd[cc][k][0] = fma(d0, qr[k][i][0], pd[cc][k][0]);
-                        pd[cc][k][1] = fma(d1, qr[k][i][1], pd[cc][k][1]);
-                    }
-                }
-            if (DIRECT) {                                        // this warp's copy of the stage is in registers: release it
-                __syncwarp();
-                if (lane == 0) mbar_arrive_cta(&empty[st]);
-            }
-            double v[CK];
-#pragma unroll
-            for (int cc = 0; cc < C; cc++)
-#pragma unroll
-                for (int k = 0; k < K; k++) v[cc * K + k] = pd[cc][k][0] + pd[cc][k][1];
-            const double sw = warp_sum_multi<CK>(v, lane);      // lanes [ck*32/CK, (ck+1)*32/CK) hold the warp total of value ck
-            if (DIRECT) {
-                const int dest = lane & (32 / CK - 1), ck = lane / (32 / CK), slot = s & 3;
-                if (dest < CS)
-                    st_async_f64(mapa_u32(smem_u32(&xbuf[slot][crank][wid][ck]), (uint32_t)dest), sw, mapa_u32(smem_u32(&full[slot]), (uint32_t)dest));
-            } else {
-                if ((lane & (32 / CK - 1)) == 0) sts_f64(red_u + (uint32_t)(((s & 3) * NCW * CK + lane / (32 / CK)) * 8), sw);
-                __syncwarp();
-                if (lane == 0) mbar_arrive_cta_u(redbar_u + 8u * (s & 3));
-            }
-        };
-        auto axpy_step = [&](const int b, int sp) {
-            const int slot = sp & 3;
-            mbar_wait_cta_u(wready_u + 8u * slot, (uint32_t)((sp >> 2) & 1));
-            double wgt[CK];
-            if constexpr (CK >= 2) {
-#pragma unroll
-                for (int i = 0; i < CK; i += 2) {
-                    const double2 w2 = lds_f64x2(wbuf_u + (uint32_t)((slot * CK + i) * 8));
-                    wgt[i] = w2.x; wgt[i + 1] = w2.y;
-                }
-            } else {
-                wgt[0] = wbuf[slot][0];
-            }
-#pragma unroll
-            for (int cc = 0; cc < C; cc++)
-#pragma unroll
-                for (int i = 0; i < RP; i++)
-#pragma unroll
-                    for (int k = 0; k < K; k++) {
-                        acc[k][i][0] = fma(a[b][cc][i][0], wgt[cc * K + k], acc[k][i][0]);
-                        acc[k][i][1] = fma(a[b][cc][i][1], wgt[cc * K + k], acc[k][i][1]);
-                    }
-        };
-        for (int s0 = 0; s0 < nsteps + DEF; s0 += DEF + 1) {
-#pragma unroll
-            for (int b = 0; b <= DEF; b++) {
-                const int s = s0 + b;
-                if (s < nsteps) dot_step(b, s);
-                if (s >= DEF && s < nsteps + DEF) axpy_step((b + 1) % (DEF + 1), s - DEF);
-            }
-        }
-#pragma unroll
-        for (int k = 0; k < K; k++) {
-            if (!active[k]) continue;
-            double* prow = partial + ((size_t)k * nchunks + blockIdx.y) * ld + rbase;
-#pragma unroll
-            for (int i = 0; i < RP; i++)
-                if (valid[i]) *reinterpret_cast<double2*>(prow + (i * CT + tid) * 2) = make_double2(acc[k][i][0], acc[k][i][1]);
-        }
-    }
-    cluster_sync_all();                                          // nobody leaves while a peer may still write into its shared memory
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// k_gram_wsx: the warp-specialised ring of k_gram_ws with the compute warps' instruction stream cut down to what the arithmetic
-// needs. The ncu capture of k_gram_ws (profiles/r02_ncu_full_k_gram_ws.txt) shows a kernel bound by issue slots and dependent
-// latencies, not by HBM: 225 instructions per compute warp and step, of which only 64 DFMA + 16 DADD are the products. The rest,
-// and where it goes here:
-//   * the 5-level shuffle butterfly over the lanes (12 SHFL + 12 FSEL + 10 MOV + 7 DADD, ~150 cycles of dependent latency per
-//     warp and step): the lanes store their CK partial sums as they are (one 16-byte store per value pair, conflict-free) and
-//     the COMMUNICATION warp adds the NCW x 32 partial sums of a value — once per CTA and step instead of once per warp;
-//   * slot, stage and parity arithmetic of the four-deep exchange: the step loop is unrolled by four, so ring stage, exchange
-//     slot and barrier are compile-time offsets from ONE shared-window base register and the parity is one bit flipped per trip;
-//   * column means: address arithmetic + LDG per column and step in every thread: the communication warp's lane 0 bulk-copies
-//     the C means of a step next to its column pieces (same mbarrier), a compute thread reads them with one broadcast LDS.128;
-//   * barrier waits: one try_wait + one branch on the fast path (the spin counter only exists on the slow path).
-// Same protocol, same summation trees across warps and ranks (so the same t_j in every CTA of a cluster); the lanes of a warp are
-// now added by the communication warp's butterfly instead of each warp's own.
-// 132 instead of 225 instructions per compute warp and step — and, measured, NOT ONE microsecond faster (2.827 ms per 17 GB shard for
-// both, to four digits; time exactly proportional to 1 / clusters; one system as slow as two): what paced k_gram_ws was not the
-// arithmetic but the refill of the ring, which sat in the communication warp's loop BEHIND the cluster round trip of the previous
-// step — a stage was re-issued one exchange latency after it had been consumed, and 3 x 40 kB in flight per SM then cover only
-// ~50 GB/s per SM (tools/tma_ingest.cu: the copy engine itself sustains 62 GB/s per SM = 7.5 TB/s on 120 SMs with the same ring).
-// PROD = 1 gives the ring its own PRODUCER warp: its lane 0 waits for the compute warps' arrival on a stage and re-issues it at
-// once, whatever the exchange is doing. 2.46 ms cold (6.9 TB/s, ncu) / 2.58-2.74 ms in bursts for two systems, 2.37 ms (7.16 TB/s,
-// the read probe's speed) for one; with the lean compute loop the issue slots are 27 % busy. An extra cp.async.bulk.prefetch.L2 ahead
-// of the ring only costs (2.76-2.93 ms): removed.
-// ---------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t opaque_u32(uint32_t x) {       // keeps the compiler from re-deriving a shared-window address (S2R + LEA) at every use
-    asm volatile("" : "+r"(x));
-    return x;
-}
-__device__ __forceinline__ bool mbar_try_cta_u(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ bool mbar_try_cluster_u(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void mbar_spin_cta_u(uint32_t bar, uint32_t parity) {
-    if (mbar_try_cta_u(bar, parity)) return;
-    uint32_t spins = 0;
-    while (!mbar_try_cta_u(bar, parity))
-        if (++spins > (1u << 28)) __trap();                      // a protocol bug must fault, not hang the GPU
-}
-__device__ __forceinline__ void mbar_spin_cluster_u(uint32_t bar, uint32_t parity) {
-    if (mbar_try_cluster_u(bar, parity)) return;
-    uint32_t spins = 0;
-    while (!mbar_try_cluster_u(bar, parity))
-        if (++spins > (1u << 28)) __trap();
-}
-__device__ __forceinline__ void mbar_init_u(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void sts_f64x2(uint32_t addr, double x, double y) {
-    asm volatile("st.shared.v2.f64 [%0], {%1,%2};" ::"r"(addr), "d"(x), "d"(y) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s_u(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-
-// Sums of NV (2 or 4) values over the lane quadruples {l, l^8, l^16, l^24}: the first two levels of warp_sum_multi. Lane l is left with the
-// quadruple's sum of value l / (32 / NV); the levels 4, 2, 1 that remain are the same for every NV.
+// Sums of NV (2 or 4) values over the lane quadruples {l, l^8, l^16, l^24}: at each level a lane hands half of its values to its
+// partner and keeps the sums of the other half, so lane l is left with the quadruple's sum of value l / (32 / NV). The levels
+// 4, 2, 1 that remain are the same for every NV; the communication warp adds them.
 template <int NV>
 __device__ __forceinline__ double quad_sum_multi(const double (&v)[NV], int lane) {
     static_assert(NV == 2 || NV == 4, "2 or 4 values");
@@ -952,42 +161,24 @@ __device__ __forceinline__ double quad_sum_multi(const double (&v)[NV], int lane
     }
 }
 
-template <int K, int NCW, int RP, int C, int CS, int PROD, int DBG = 0, int RED = 0>
-__global__ void __launch_bounds__((NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) * 32, 1) k_gram_wsx(const double* __restrict__ A, size_t ld, const double* __restrict__ mave,
-                                                               const double* __restrict__ msig, GramVec gv, int tile_rows, int cols_per_chunk,
-                                                               long long M, double scale, double* __restrict__ partial, int nchunks,
-                                                               const __grid_constant__ CUtensorMap tmap) {
-    constexpr bool TENSOR = PROD >= 2;                           // one tensor copy per step (all C column pieces) instead of C + 1 bulk copies
-    // PROD = 3: the service warps form a warpgroup of their own (communication warp, producer warp, two idle warps) that hands its
-    // registers to the compute warpgroups (setmaxnreg): 8 compute warps x 5 row pairs need ~200 registers, and a CTA of 10 warps is
-    // allotted registers as if it had 12 (168 per thread) — with two compute warps on every scheduler instead of 3 / 3 / 2 / 2
-    constexpr bool REALLOC = PROD == 3;
-    // DBG 3: cluster 0's rank 0 writes clock64() stamps of every hand-over of its first 3000 steps into t[0] (32 slots per step) instead of the
-    // products (tools/gram_trace.py reads them back); wrong results, timing experiments only
-    long long* const trace = DBG == 3 && blockIdx.y == 0 ? reinterpret_cast<long long*>(gv.t[0]) : nullptr;
-    auto stamp = [&](int s, int slot) {
-        if (DBG == 3) {
-            uint32_t cr;
-            asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(cr));
-            if (trace != nullptr && cr == 0 && s < 3000 && (threadIdx.x & 31) == 0) trace[s * 32 + slot] = clock64();
-        }
-    };
-    static_assert(!REALLOC || NCW % 4 == 0, "whole warpgroups of compute warps");
-    constexpr int R = 4, CK = C * K, NPAIR = CK / 2, LPV = 32 / CK, CT = NCW * 32, PIECE = CT * RP * 2;
-    static_assert(C == 2 && (K == 1 || K == 2), "two columns per step: their means are one 16-byte bulk copy, their sums one or two value pairs");
+// K systems (1 or 2), CS CTAs per cluster (1 ... 16). Warps 0 ... NCW-1 compute; warp NCW communicates, warp NCW+1 produces.
+template <int K, int CS>
+__global__ void __launch_bounds__(GRAM_THREADS, 1) k_gram_wsx(const double* __restrict__ A, size_t ld, const double* __restrict__ mave,
+                                                             const double* __restrict__ msig, GramVec gv, int tile_rows, int cols_per_chunk,
+                                                             long long M, double scale, double* __restrict__ partial, int nchunks,
+                                                             const __grid_constant__ CUtensorMap tmap) {
+    constexpr int NCW = GRAM_NCW, RP = GRAM_RP, C = GRAM_C, R = GRAM_R;
+    constexpr int CK = C * K, LPV = 32 / CK, CT = NCW * 32, PIECE = CT * RP * 2;
+    static_assert(C == 2 && (K == 1 || K == 2), "two columns per step: their means are one 16-byte load, their sums one or two value pairs");
     static_assert(CS <= 2 * LPV, "after the butterfly the LPV lanes that hold value ck send it to the CS ranks, at most two each");
     // one control block, addressed as base register + compile-time offset (bytes)
     constexpr uint32_t XSLOT = CS * CK * 8;                      // xbuf[4][CS][CK]: partial sums of the ranks, per exchange slot
     constexpr uint32_t XBUF_O = 0, WBUF_O = XBUF_O + 4 * XSLOT;  // wbuf[4][CK]: axpy weights of a step
     constexpr uint32_t MST_O = WBUF_O + 4 * CK * 8;              // mst[R][C]: column means of a ring stage
     constexpr uint32_t FULL_O = MST_O + R * C * 8, WREADY_O = FULL_O + 32, REDBAR_O = WREADY_O + 32, RINGBAR_O = REDBAR_O + 32;
-    // RED = 0: red[2][NCW][NPAIR][32 lanes] value pairs — the lanes' sums as they are, the communication warp adds warps and lanes;
-    // RED = 1: red[2][NCW][32 lanes] — every compute warp first adds its lane quadruples (two shuffle levels, hidden in the time the
-    //          warp waits for the previous step's weights anyway), the communication warp adds the warps and the three levels left.
-    //          The time stamps of shape 15 (tools/gram_trace.py) show the communication warp to be the step's critical path:
-    //          ~670 of its ~1180 cycles per step went into reading and adding the 10 x 32 x 4 lane sums
+    // red[2][NCW][32 lanes]: every compute warp's quadruple sums, as they are
     constexpr uint32_t RED_O = RINGBAR_O + R * 8;
-    constexpr uint32_t REDSLOT = RED ? NCW * 256 : NCW * NPAIR * 512, CTL_BYTES = RED_O + 2 * REDSLOT;
+    constexpr uint32_t REDSLOT = NCW * 256, CTL_BYTES = RED_O + 2 * REDSLOT;
     static_assert(RED_O % 16 == 0, "16-byte stores");
     extern __shared__ __align__(128) double ring[];              // [R][C][PIECE]
     __shared__ __align__(16) unsigned char ctl[CTL_BYTES];
@@ -995,7 +186,7 @@ __global__ void __launch_bounds__((NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) *
     bool any = false;
 #pragma unroll
     for (int k = 0; k < K; k++) { active[k] = gv.done[k] == nullptr || *gv.done[k] == 0; any |= active[k]; }
-    if (!any) return;
+    if (!any) return;                                            // identical decision in every CTA of the cluster
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     uint32_t crank;
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(crank));
@@ -1003,24 +194,18 @@ __global__ void __launch_bounds__((NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) *
     const long long c0 = (long long)blockIdx.y * cols_per_chunk;
     long long c1 = c0 + cols_per_chunk;
     if (c1 > M) c1 = M;
+    // steps and column offsets are 32-bit: a chunk has far fewer than 2^31 columns
     const int ncols = c1 > c0 ? (int)(c1 - c0) : 0;
     const int nsteps = (ncols + C - 1) / C;
-    const uint32_t piece_bytes = rbase < ld ? (uint32_t)((ld - rbase < (size_t)tile_rows ? ld - rbase : (size_t)tile_rows) * sizeof(double)) : 0u;
     const double* const mave_c = mave + c0;
     const double* const msig_c = msig + c0;
-    auto col_of = [&](int s, int cc) { const int j = s * C + cc; return j < ncols ? j : ncols - 1; };
-    // rows of the ring slots that no bulk copy ever writes are zeroed once (see k_gram_ws)
-    if (TENSOR) {
-        // a stage holds the C column pieces back to back, tile_rows rows each (rows past the end of the column arrive as zeros: the
-        // copy engine fills what lies outside the tensor); the stage's tail behind them is never written
-        for (int i = C * tile_rows + tid; i < C * PIECE; i += blockDim.x)
+    auto col_of = [&](int s, int cc) { const int j = s * C + cc; return j < ncols ? j : ncols - 1; };   // ragged last step: its last column again
+    // a stage holds the C column pieces back to back, tile_rows rows each; the stage's tail behind them is never written by a copy,
+    // so it is zeroed once: every compute thread can then load its row pairs unconditionally — a zero row has q = 0 and its w is
+    // never stored
+    for (int i = C * tile_rows + tid; i < C * PIECE; i += blockDim.x)
 #pragma unroll
-            for (int st = 0; st < R; st++) ring[(size_t)st * C * PIECE + i] = 0.0;
-    } else {
-        for (int i = (int)(piece_bytes / 8) + tid; i < PIECE; i += blockDim.x)
-#pragma unroll
-            for (int sc = 0; sc < R * C; sc++) ring[(size_t)sc * PIECE + i] = 0.0;
-    }
+        for (int st = 0; st < R; st++) ring[(size_t)st * C * PIECE + i] = 0.0;
     const uint32_t cb = opaque_u32(smem_u32(ctl)), ring_u = opaque_u32(smem_u32(ring));
     if (tid == 0) {
 #pragma unroll
@@ -1036,32 +221,11 @@ __global__ void __launch_bounds__((NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) *
     cluster_sync_all();                                          // every CTA's mbarriers are armed before anybody sends
 
     if (wid >= NCW) {
-        // ------------------------- communication warp (and, with PROD, the ring's producer warp) -------------------------
-        if (REALLOC) asm volatile("setmaxnreg.dec.sync.aligned.u32 96;");
-        const double* const a_c = A + rbase + (size_t)c0 * ld;
-        const bool m_aligned = (reinterpret_cast<uintptr_t>(mave_c) & 15) == 0;
-        auto issue_step = [&](int s, int st) {                   // lane 0: the C column pieces and means of step s into stage st = s % 4
-            const uint32_t bar = cb + RINGBAR_O + 8 * st;
-            const bool mb = m_aligned && s * C + C <= ncols;     // a ragged last step repeats its last column: means written by hand
-            if (!mb) {
-#pragma unroll
-                for (int cc = 0; cc < C; cc++) sts_f64(cb + MST_O + (uint32_t)((st * C + cc) * 8), __ldg(mave_c + col_of(s, cc)));
-            }
-            mbar_expect_tx_u(bar, C * piece_bytes + (mb ? C * 8u : 0u));
-            if (mb) bulk_g2s_u(cb + MST_O + (uint32_t)(st * C * 8), mave_c + s * C, C * 8, bar);
-            if (piece_bytes != 0) {
-#pragma unroll
-                for (int cc = 0; cc < C; cc++)
-                    bulk_g2s_u(ring_u + (uint32_t)((st * C + cc) * PIECE * 8), a_c + (size_t)col_of(s, cc) * ld, piece_bytes, bar);
-            }
-        };
-        if (TENSOR && wid == NCW + 1) {
-            // producer warp, tensor form: ONE cp.async.bulk.tensor per step brings all C column pieces (box 16 x tile_rows/16 x C of the
-            // {16, ld/16, M} view of the marker block). A warp gets one bulk copy of any size under way every ~500-650 cycles
-            // (tools/tma_ingest2.cu: the rate scales with the number of ISSUING WARPS, not with bytes or copies in flight), so the
-            // C + 1 copies per step of the PROD = 1 form cost the producer ~1300 cycles per step — exactly what that form measures
-            // per step at any clock and any number of clusters (profiles/r02_gram_sustained_clock.jsonl). The column means travel
-            // beside the copy: lanes < C fetch them before waiting for the stage and store them before lane 0 arrives on its barrier.
+        // ----------------------------------------------- service warpgroup -----------------------------------------------
+        asm volatile("setmaxnreg.dec.sync.aligned.u32 96;");
+        if (wid == NCW + 1) {
+            // producer warp. The column means travel beside the copy: lanes < C fetch them before waiting for the stage and store
+            // them before lane 0 arrives on its barrier.
             const int row16 = (int)(rbase >> 4), box_bytes = C * tile_rows * 8;
             auto issue_tensor = [&](int s, int st, double mv) {
                 if (lane < C) sts_f64(cb + MST_O + (uint32_t)((st * C + lane) * 8), mv);
@@ -1086,103 +250,64 @@ __global__ void __launch_bounds__((NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) *
                     issue_tensor(s + R, u, mv);
                 }
             }
-        } else if (!TENSOR && lane == 0 && wid == NCW + (PROD ? 1 : 0)) {
-            for (int s = 0; s < R && s < nsteps; s++) issue_step(s, s);
         }
-        if ((TENSOR && wid == NCW + 1) || (REALLOC && wid > NCW + 1)) {
-        } else if (!TENSOR && PROD && wid == NCW + 1) {
-            // producer warp: refills a ring stage the moment every compute warp has consumed it, however far the communication warp's
-            // exchange of that step has got (as part of the communication warp's loop the refill waited for the previous step's
-            // cluster round trip)
-            if (lane == 0) {
-                uint32_t php = 0;
-                for (int s0 = 0; s0 + R < nsteps; s0 += 4, php ^= 1u) {
+        if (wid <= NCW) {
+            // communication warp: wid == NCW (warps NCW + 2 and NCW + 3 only hand their registers over)
+            const int ck = lane / LPV, dst = lane % LPV, cc_l = ck / K, k_l = ck % K;   // after the butterfly lanes [ck*LPV, (ck+1)*LPV) hold value ck
+            bool act = active[0];
 #pragma unroll
-                    for (int u = 0; u < 4; u++) {
-                        const int s = s0 + u;
-                        if (s + R >= nsteps) break;
-                        mbar_spin_cta_u(cb + REDBAR_O + 8 * u, php);
-                        issue_step(s + R, u);
-                    }
-                }
-            }
-        } else {
-        const int ck = lane / LPV, dst = lane % LPV, cc_l = ck / K, k_l = ck % K;   // after the butterfly lanes [ck*LPV, (ck+1)*LPV) hold value ck
-        bool act = active[0];
+            for (int k = 1; k < K; k++) act = k_l == k ? active[k] : act;
+            double* tout = K > 1 && k_l == 1 ? gv.t[K - 1] : gv.t[0];
+            double sg_next = nsteps > 0 ? __ldg(msig_c + col_of(0, cc_l)) : 0.0;
+            const uint32_t peer = (uint32_t)(dst < CS ? dst : 0), peer2 = (uint32_t)(dst + LPV < CS ? dst + LPV : 0);   // 16-CTA clusters: two ranks per lane
+            const uint32_t rx = mapa_u32(cb + XBUF_O + (crank * CK + ck) * 8, peer), rf = mapa_u32(cb + FULL_O, peer);
+            const uint32_t rx2 = mapa_u32(cb + XBUF_O + (crank * CK + ck) * 8, peer2), rf2 = mapa_u32(cb + FULL_O, peer2);
+            const uint32_t xb_l = cb + XBUF_O + (uint32_t)ck * 8u, wb_l = cb + WBUF_O + (uint32_t)ck * 8u;
+            uint32_t ph = 0;                                     // (s / 4) & 1: phase parity of every four-deep barrier ring
+            for (int s0 = 0; s0 < nsteps; s0 += 4, ph ^= 1u) {
 #pragma unroll
-        for (int k = 1; k < K; k++) act = k_l == k ? active[k] : act;
-        double* tout = K > 1 && k_l == 1 ? gv.t[K - 1] : gv.t[0];
-        double sg_next = nsteps > 0 ? __ldg(msig_c + col_of(0, cc_l)) : 0.0;
-        const uint32_t peer = (uint32_t)(dst < CS ? dst : 0), peer2 = (uint32_t)(dst + LPV < CS ? dst + LPV : 0);   // 16-CTA clusters: two ranks per lane
-        const uint32_t rx = mapa_u32(cb + XBUF_O + (crank * CK + ck) * 8, peer), rf = mapa_u32(cb + FULL_O, peer);
-        const uint32_t rx2 = mapa_u32(cb + XBUF_O + (crank * CK + ck) * 8, peer2), rf2 = mapa_u32(cb + FULL_O, peer2);
-        const uint32_t red_l = cb + RED_O + (uint32_t)lane * 16u, xb_l = cb + XBUF_O + (uint32_t)ck * 8u, wb_l = cb + WBUF_O + (uint32_t)ck * 8u;
-        uint32_t ph = 0;                                         // (s / 4) & 1: phase parity of every four-deep barrier ring
-        for (int s0 = 0; s0 < nsteps; s0 += 4, ph ^= 1u) {
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-                const int s = s0 + u;
-                if (s >= nsteps) break;
-                const double sgl = sg_next;
-                sg_next = __ldg(msig_c + col_of(s + 1 < nsteps ? s + 1 : s, cc_l));
-                mbar_spin_cta_u(cb + REDBAR_O + 8 * u, ph);       // every compute warp has read stage u and stored its partial sums
-                stamp(s, 24);
-                if (!PROD && lane == 0 && s + R < nsteps) issue_step(s + R, u);
-                double sw;                                       // the CTA's partial sum of value ck
-                if constexpr (RED == 1) {
+                for (int u = 0; u < 4; u++) {
+                    const int s = s0 + u;
+                    if (s >= nsteps) break;
+                    const double sgl = sg_next;
+                    sg_next = __ldg(msig_c + col_of(s + 1 < nsteps ? s + 1 : s, cc_l));
+                    mbar_spin_cta_u(cb + REDBAR_O + 8 * u, ph);   // every compute warp has read stage u and stored its partial sums
+                    // the CTA's partial sum of value ck: the warps by a fixed tree, then the lane levels 4, 2, 1
                     double pw[NCW];
 #pragma unroll
                     for (int w = 0; w < NCW; w++) pw[w] = lds_f64(cb + RED_O + (uint32_t)((u & 1) * REDSLOT + w * 256) + (uint32_t)lane * 8u);
-                    sw = tree_sum<NCW>(pw);
+                    double sw = tree_sum<NCW>(pw);
                     sw += __shfl_xor_sync(0xffffffffu, sw, 4);
                     sw += __shfl_xor_sync(0xffffffffu, sw, 2);
                     sw += __shfl_xor_sync(0xffffffffu, sw, 1);
-                } else {
-                double vs[CK];                                   // this lane's sum over the warps (fixed tree) of its slice of every value
+                    if (dst < CS) st_async_f64(rx + u * XSLOT, sw, rf + 8 * u);
+                    if (CS > LPV && dst + LPV < CS) st_async_f64(rx2 + u * XSLOT, sw, rf2 + 8 * u);
+                    // the ranks' values arrive as st.async transactions ON this barrier (data and count are one message), so the
+                    // CTA-scope wait orders them; the cluster-scope acquire form would cost an L1 invalidation (CCTL.IVALL) per step
+                    mbar_spin_cta_u(cb + FULL_O + 8 * u, ph);
+                    // every lane adds the CS partial sums of its value by the same fixed tree: bitwise the same t_j in every CTA
+                    double pr[CS];
 #pragma unroll
-                for (int pr = 0; pr < NPAIR; pr++) {
-                    double px[NCW], py[NCW];
-#pragma unroll
-                    for (int w = 0; w < NCW; w++) {
-                        const double2 x = DBG == 2 && w > 0 ? make_double2(px[0] + 1.0, py[0] + 1.0) : lds_f64x2(red_l + (uint32_t)((u & 1) * REDSLOT + (w * NPAIR + pr) * 512));
-                        px[w] = x.x; py[w] = x.y;
+                    for (int r = 0; r < CS; r++) pr[r] = lds_f64(xb_l + (uint32_t)(u * XSLOT + r * CK * 8));
+                    const double tot = tree_sum<CS>(pr);
+                    const int j = s * C + cc_l;
+                    const double tj = (sgl * tot) * scale;                      // sigma_inv * dpa (:306), then * scale (:330)
+                    const bool live = j < ncols && act;
+                    if (dst == 0) {
+                        if (crank == 0 && live) tout[c0 + j] = tj;
+                        sts_f64(wb_l + (uint32_t)(u * CK * 8), live ? sgl * tj : 0.0);   // sig_phen_i = msig * x, src/data.cpp:354
                     }
-                    vs[2 * pr] = tree_sum<NCW>(px); vs[2 * pr + 1] = tree_sum<NCW>(py);
+                    __syncwarp();
+                    if (lane == 0) {
+                        mbar_arrive_cta_u(cb + WREADY_O + 8 * u);
+                        mbar_expect_tx_u(cb + FULL_O + 8 * u, XSLOT);           // re-arm the slot for step s + 4
+                    }
                 }
-                sw = warp_sum_multi<CK>(vs, lane);
-                }
-                if (dst < CS) st_async_f64(rx + u * XSLOT, sw, rf + 8 * u);
-                if (CS > LPV && dst + LPV < CS) st_async_f64(rx2 + u * XSLOT, sw, rf2 + 8 * u);
-                stamp(s, 25);
-                // the ranks' values arrive as st.async transactions ON this barrier (data and count are one message), so the CTA-scope wait
-                // orders them; the cluster-scope acquire form costs a CCTL.IVALL (L1 invalidation) per step — 14 % of this warp's time in
-                // the ncu samples of shape 10 — that shared memory does not need
-                if (TENSOR) mbar_spin_cta_u(cb + FULL_O + 8 * u, ph); else mbar_spin_cluster_u(cb + FULL_O + 8 * u, ph);
-                stamp(s, 26);
-                // every lane adds the CS partial sums of its value by the same fixed tree: bitwise the same t_j in every CTA
-                double pr[CS];
-#pragma unroll
-                for (int r = 0; r < CS; r++) pr[r] = lds_f64(xb_l + (uint32_t)(u * XSLOT + r * CK * 8));
-                const double tot = tree_sum<CS>(pr);
-                const int j = s * C + cc_l;
-                const double tj = (sgl * tot) * scale;                          // sigma_inv * dpa (:306), then * scale (:330)
-                const bool live = j < ncols && act;
-                if (dst == 0) {
-                    if (live && crank == 0 && DBG != 3) tout[c0 + j] = tj;
-                    sts_f64(wb_l + (uint32_t)(u * CK * 8), live ? sgl * tj : 0.0);   // sig_phen_i = msig * x, src/data.cpp:354
-                }
-                __syncwarp();
-                if (lane == 0) {
-                    mbar_arrive_cta_u(cb + WREADY_O + 8 * u);
-                    mbar_expect_tx_u(cb + FULL_O + 8 * u, XSLOT);               // re-arm the slot for step s + 4
-                }
-                stamp(s, 27);
             }
-        }
         }
     } else {
         // ---------------------------------------------- compute warps ----------------------------------------------
-        if (REALLOC) asm volatile("setmaxnreg.inc.sync.aligned.u32 200;");
+        asm volatile("setmaxnreg.inc.sync.aligned.u32 200;");
         bool valid[RP];
         double qr[K][RP][2], acc[K][RP][2];
 #pragma unroll
@@ -1198,9 +323,8 @@ __global__ void __launch_bounds__((NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) *
             }
         }
         double a[2][C][RP][2];                                   // the step being dotted and the step whose axpy is pending
-        const uint32_t rows_u = opaque_u32(ring_u + (uint32_t)tid * 16u);             // this thread's first row pair inside a ring slot
-        const uint32_t col_stride = TENSOR ? (uint32_t)tile_rows * 8u : (uint32_t)PIECE * 8u;   // bytes between the column pieces of a stage
-        const uint32_t red_w = opaque_u32(cb + RED_O + (uint32_t)(wid * NPAIR) * 512u + (uint32_t)lane * 16u);
+        const uint32_t rows_u = opaque_u32(ring_u + (uint32_t)tid * 16u);             // this thread's first row pair inside a ring stage
+        const uint32_t col_stride = (uint32_t)tile_rows * 8u;                         // bytes between the column pieces of a stage
 
         auto dot_step = [&](const int u, const uint32_t par, const int s) {   // u = s % 4: ring stage, barrier; u & 1: register buffer, red slot
             double pd[C][K][2];
@@ -1208,19 +332,15 @@ __global__ void __launch_bounds__((NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) *
             for (int cc = 0; cc < C; cc++)
 #pragma unroll
                 for (int k = 0; k < K; k++) pd[cc][k][0] = pd[cc][k][1] = 0.0;
-            if (wid == 0) stamp(s, 20);
             mbar_spin_cta_u(cb + RINGBAR_O + 8 * u, par);
-            if (wid == 0) stamp(s, 21);
             const double2 mm = lds_f64x2(cb + MST_O + (uint32_t)(u * C * 8));
             const double m[2] = {mm.x, mm.y};
 #pragma unroll
             for (int cc = 0; cc < C; cc++)
 #pragma unroll
                 for (int i = 0; i < RP; i++) {
-                    // rows beyond the tile read zeros (tensor form: or the next column's first rows — they only meet q = 0 and unsaved sums)
-                    // DBG (timing experiments only, wrong results): 1 = the second column of a step is not read from shared memory
-                    const double2 v = DBG == 1 && cc > 0 ? make_double2(a[u & 1][0][i][0] + m[0], a[u & 1][0][i][1] + m[0])
-                                                         : lds_f64x2(rows_u + (uint32_t)((u * C * PIECE + i * CT * 2) * 8) + (uint32_t)cc * col_stride);
+                    // rows beyond the tile read zeros or the next column's first rows: they only meet q = 0 and unsaved sums
+                    const double2 v = lds_f64x2(rows_u + (uint32_t)((u * C * PIECE + i * CT * 2) * 8) + (uint32_t)cc * col_stride);
                     const double d0 = v.x - m[cc], d1 = v.y - m[cc];            // meth[i] - mu, src/data.cpp:304 and :360
                     a[u & 1][cc][i][0] = d0; a[u & 1][cc][i][1] = d1;           // kept centred for the deferred axpy
 #pragma unroll
@@ -1234,20 +354,12 @@ __global__ void __launch_bounds__((NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) *
             for (int cc = 0; cc < C; cc++)
 #pragma unroll
                 for (int k = 0; k < K; k++) v[cc * K + k] = pd[cc][k][0] + pd[cc][k][1];
-            if constexpr (RED == 1) {
-                sts_f64(cb + RED_O + (uint32_t)((u & 1) * REDSLOT + wid * 256) + (uint32_t)lane * 8u, quad_sum_multi<CK>(v, lane));
-            } else {
-#pragma unroll
-            for (int pr = 0; pr < NPAIR; pr++)
-                if (DBG != 2 || v[2 * pr] == 123.456) sts_f64x2(red_w + (uint32_t)((u & 1) * REDSLOT + pr * 512), v[2 * pr], v[2 * pr + 1]);   // DBG 2: partial sums never stored
-            }
+            sts_f64(cb + RED_O + (uint32_t)((u & 1) * REDSLOT + wid * 256) + (uint32_t)lane * 8u, quad_sum_multi<CK>(v, lane));
             __syncwarp();
             if (lane == 0) mbar_arrive_cta_u(cb + REDBAR_O + 8 * u);
-            stamp(s, wid);
         };
-        auto axpy_step = [&](const int slot, const uint32_t par, const int b, const int s) {
+        auto axpy_step = [&](const int slot, const uint32_t par, const int b) {
             mbar_spin_cta_u(cb + WREADY_O + 8 * slot, par);
-            stamp(s, 10 + wid);
             double wgt[CK];
 #pragma unroll
             for (int i = 0; i < CK; i += 2) {
@@ -1270,7 +382,7 @@ __global__ void __launch_bounds__((NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) *
             for (int u = 0; u < 4; u++) {
                 const int s = s0 + u;
                 if (s < nsteps) dot_step(u, ph, s);
-                if (s >= 1 && s <= nsteps) axpy_step((u + 3) & 3, u == 0 ? ph ^ 1u : ph, (u + 1) & 1, s - 1);   // step s - 1
+                if (s >= 1 && s <= nsteps) axpy_step((u + 3) & 3, u == 0 ? ph ^ 1u : ph, (u + 1) & 1);   // step s - 1
             }
         }
 #pragma unroll
@@ -1285,57 +397,6 @@ __global__ void __launch_bounds__((NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) *
     cluster_sync_all();                                          // nobody leaves while a peer may still write into its shared memory
 }
 
-template <int K, int C, int CS, typename Kern, typename... Extra>
-int gram_launch_any(vampomi_ctx* c, Kern kern, int TPB, int ROWS, size_t smem, int shape, const GramVec& gv, const MultiVec& mw, Extra... extra) {
-    const size_t tr = (c->ld + CS - 1) / CS;
-    const int tile_rows = (int)((tr + 15) / 16 * 16);
-    if (tile_rows > ROWS) { set_error("gram: N=%d needs more than %d rows per CTA at cluster size %d", c->N, ROWS, CS); return VAMPOMI_ERR_ARG; }
-    cudaLaunchConfig_t cfg = {};
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CS; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.blockDim = dim3(TPB); cfg.dynamicSmemBytes = smem; cfg.stream = c->stream; cfg.attrs = attr; cfg.numAttrs = 1;
-    // co-resident clusters of this (shape, cluster size, systems) on this device: queried once per context
-    static_assert(CS >= 1 && CS <= 16, "cluster size");
-    int& ncl = c->gram_clusters[shape][CS][K - 1];
-    if (ncl <= 0) {
-        if (smem > 40 * 1024) VO_CUDA(cudaFuncSetAttribute((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        if (CS > 8) VO_CUDA(cudaFuncSetAttribute((const void*)kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));   // 16 CTAs: one cluster per GPC
-        cfg.gridDim = dim3(CS, c->num_sms);
-        int n = 0;
-        if (cudaOccupancyMaxActiveClusters(&n, (const void*)kern, &cfg) != cudaSuccess || n < 1) { cudaGetLastError(); n = c->num_sms / CS; }
-        ncl = n < 1 ? 1 : n;
-    }
-    long long nch = c->tune.gram_clusters > 0 ? c->tune.gram_clusters : ncl;
-    const long long cap = (c->M + C - 1) / C;
-    if (nch > cap) nch = cap;
-    int cols_per_chunk = (int)((c->M + nch - 1) / nch);
-    cols_per_chunk = (cols_per_chunk + C - 1) / C * C;
-    const int nchunks = (int)((c->M + cols_per_chunk - 1) / cols_per_chunk);
-    VO_CHECK(ensure_ax_partial(c, (size_t)K * nchunks * c->ld));
-    cfg.gridDim = dim3(CS, nchunks);
-    if (c->prof_pending.size() > 8192) VO_CHECK(prof_resolve(c));
-    int sp = prof_begin(c, 3, (double)c->M * c->N * (double)c->elem_bytes);
-    const double scale = 1.0 / sqrt((double)c->N);
-    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, (const double*)c->A, c->ld, (const double*)c->mave, (const double*)c->msig, gv, tile_rows,
-                                       cols_per_chunk, c->M, scale, c->ax_partial, nchunks, extra...);
-    prof_end(c, sp);
-    if (e != cudaSuccess) { set_error("gram kernel launch failed: %s", cudaGetErrorString(e)); cudaGetLastError(); return VAMPOMI_ERR_CUDA; }
-    c->counters[0] += 1; c->counters[1]++; c->counters[2] += (long long)c->M * c->N * c->elem_bytes;
-    return launch_ax_reduce_multi(c, nchunks, mw);
-}
-
-template <int K, int TPB, int RV, int C, int D, int CS, int QS>
-int gram_launch(vampomi_ctx* c, const GramVec& gv, const MultiVec& mw, int shape) {
-    constexpr int ROWS = TPB * RV * 4;
-    return gram_launch_any<K, C, CS>(c, k_gram<K, TPB, RV, C, D, CS, QS>, TPB, ROWS, QS ? (size_t)K * ROWS * sizeof(double) : 0, shape, gv, mw,
-                                     c->tune.gram_prefetch);
-}
-template <int K, int NCW, int RP, int C, int R, int CS, int DIRECT, int DEF = 1, int NCOMM = 1>
-int gram_launch_ws(vampomi_ctx* c, const GramVec& gv, const MultiVec& mw, int shape) {
-    constexpr int ROWS = NCW * 32 * RP * 2;
-    return gram_launch_any<K, C, CS>(c, k_gram_ws<K, NCW, RP, C, R, CS, DIRECT, DEF, NCOMM>, (NCW + NCOMM) * 32, ROWS, (size_t)R * C * ROWS * sizeof(double), shape, gv, mw);
-}
 // {16, ld/16, M} view of the column-major marker block (a column = ld/16 groups of 16 rows) with a box of one CTA's row tile of C
 // columns: 16 x tile_rows/16 x C doubles land in shared memory as C contiguous column pieces. Cached in the context.
 int gram_tensor_map(vampomi_ctx* c, int tile_rows, int C, CUtensorMap* out) {
@@ -1366,126 +427,53 @@ int gram_tensor_map(vampomi_ctx* c, int tile_rows, int C, CUtensorMap* out) {
     return VAMPOMI_OK;
 }
 
-template <int K, int NCW, int RP, int C, int CS, int PROD, int DBG = 0, int RED = 0>
-int gram_launch_wsx(vampomi_ctx* c, const GramVec& gv, const MultiVec& mw, int shape) {
-    constexpr int ROWS = NCW * 32 * RP * 2;
-    if constexpr (CS <= 2 * (32 / (C * K))) {
-        CUtensorMap tm;
-        memset(&tm, 0, sizeof(tm));
-        if (PROD >= 2) {
-            const size_t tr = (c->ld + CS - 1) / CS;
-            VO_CHECK(gram_tensor_map(c, (int)((tr + 15) / 16 * 16), C, &tm));
-        }
-        return gram_launch_any<K, C, CS>(c, k_gram_wsx<K, NCW, RP, C, CS, PROD, DBG, RED>, (NCW + (PROD == 3 ? 4 : 1 + (PROD ? 1 : 0))) * 32, ROWS, (size_t)4 * C * ROWS * sizeof(double), shape, gv, mw, tm);
-    } else {
-        set_error("gram: shape %d holds at most %d CTAs per cluster", shape, 2 * (32 / (C * K)));
-        return VAMPOMI_ERR_ARG;
-    }
-}
-template <int K, int TPB, int RP, int C, int R, int CS>
-int gram_launch_bulk(vampomi_ctx* c, const GramVec& gv, const MultiVec& mw, int shape) {
-    constexpr int ROWS = TPB * RP * 2;
-    return gram_launch_any<K, C, CS>(c, k_gram_bulk<K, TPB, RP, C, R, CS>, TPB, ROWS, (size_t)R * C * ROWS * sizeof(double), shape, gv, mw);
-}
-
-// shapes (knob gram_shape)
-//   register-staged (k_gram): threads, 32-byte vectors per thread, columns per step, register buffers, q in shared memory
-//     0  320, 2, 2, 3, smem    1  256, 3, 2, 3, smem    2  320, 2, 2, 2, regs
-//   bulk-copy ring (k_gram_bulk): threads, 16-byte row pairs per thread, columns per step, ring stages
-//     3  256, 5, 2, 4          4  256, 5, 2, 3          5  256, 5, 1, 6
-//   warp-specialised bulk-copy ring (k_gram_ws): compute warps, row pairs per thread, columns per step, ring stages
-//     6  10, 4, 2, 4           7  the same, every compute warp sending its own partial sums (no block-level stage)
-//     8  10, 2, 4, 4: half the rows per CTA (16 CTAs per cluster at N = 20 000, one cluster per GPC) and FOUR columns per step, so the
-//        cluster round trip of a step (~0.6 us) is shorter than the step's own HBM time (80 kB per SM pair ... 40 kB per SM: 0.7 us)
-//        (measured, profiles/r02_sweep_gram_kernel_shapes.jsonl: 3.9 ms against 3.1 ms of shape 6; deferring the axpy by two steps
-//        (DEF = 2) and separate sender / receiver warps (NCOMM = 2) changed nothing there — 3.9 / 3.8 ms — so those variants are
-//        not instantiated: with DEF = 2 the four exchange slots would also have to become eight)
-//     9  k_gram_wsx: shape 6 with the lean compute loop (lane sums in the communication warp, 4x unrolled step loop, column means by
-//        bulk copy)   10  the same with a producer warp for the ring
-//    11  shape 10 with ONE tensor copy per step (cp.async.bulk.tensor.3d: both column pieces) instead of three bulk copies (default)
-//    12  shape 11 with 8 compute warps x 5 row pairs — two compute warps on every scheduler (10 leave two schedulers with three) — and a
-//        service warpgroup that hands its registers to the compute warpgroups (setmaxnreg 96 / 200: the pool is the 384 x 168 registers the CTA was launched with)
-//     (14 compute warps x 3 row pairs — 15 warps per SM under a 128-register cap — measured 3.35-3.45 ms against 3.08-3.30 of shape 6
-//     on the same box: more warps do not pay for the smaller register budget; not instantiated)
-constexpr int gram_rows_of_shape(int shape) { return shape == 1 ? 3072 : shape == 8 ? 1280 : 2560; }
-constexpr int gram_max_cluster_of_shape(int shape) { return shape == 8 || shape == 11 || shape == 12 || shape == 16 || shape == 18 ? 16 : 8; }   // 16: non-portable cluster size, one cluster per GPC
-
 template <int K, int CS>
-int gram_shape(vampomi_ctx* c, const GramVec& gv, const MultiVec& mw, int shape) {
-    switch (shape) {
-        case 0: return gram_launch<K, 320, 2, 2, 3, CS, 1>(c, gv, mw, shape);
-        case 1: return gram_launch<K, 256, 3, 2, 3, CS, 1>(c, gv, mw, shape);
-        case 2: return gram_launch<K, 320, 2, 2, 2, CS, 0>(c, gv, mw, shape);
-        case 3: return gram_launch_bulk<K, 256, 5, 2, 4, CS>(c, gv, mw, shape);
-        case 4: return gram_launch_bulk<K, 256, 5, 2, 3, CS>(c, gv, mw, shape);
-        case 5: return gram_launch_bulk<K, 256, 5, 1, 6, CS>(c, gv, mw, shape);
-        case 6: return gram_launch_ws<K, 10, 4, 2, 4, CS, 0>(c, gv, mw, shape);
-        case 7: return gram_launch_ws<K, 10, 4, 2, 4, CS, 1>(c, gv, mw, shape);
-        case 8: return gram_launch_ws<K, 10, 2, 4, 4, CS, 0>(c, gv, mw, shape);
-        case 9: return gram_launch_wsx<K, 10, 4, 2, CS, 0>(c, gv, mw, shape);
-        case 10: return gram_launch_wsx<K, 10, 4, 2, CS, 1>(c, gv, mw, shape);
-        case 11: return gram_launch_wsx<K, 10, 4, 2, CS, 2>(c, gv, mw, shape);
-        case 12: return gram_launch_wsx<K, 8, 5, 2, CS, 3>(c, gv, mw, shape);
-        case 16: return gram_launch_wsx<K, 10, 4, 2, CS, 2, 0, 1>(c, gv, mw, shape);
-        case 18: break;                                          // shape 12's warp layout with shape 16's sums: gram_cluster() (any cluster size)
-#ifdef VAMPOMI_GRAM_EXPERIMENTS
-        // timing experiments with deliberately WRONG results — not in the product library: make EXTRA_NVFLAGS=-DVAMPOMI_GRAM_EXPERIMENTS
-        case 13: if constexpr (CS == 8) return gram_launch_wsx<K, 10, 4, 2, CS, 2, 1>(c, gv, mw, shape); else break;
-        case 14: if constexpr (CS == 8) return gram_launch_wsx<K, 10, 4, 2, CS, 2, 2>(c, gv, mw, shape); else break;
-        case 15: if constexpr (CS == 8) return gram_launch_wsx<K, 10, 4, 2, CS, 2, 3>(c, gv, mw, shape); else break;   // hand-over time stamps (tools/gram_trace.py)
-        case 17: if constexpr (CS == 8) return gram_launch_wsx<K, 10, 4, 2, CS, 2, 3, 1>(c, gv, mw, shape); else break;   // shape 16 with time stamps
-#endif
-        default: break;
+int gram_launch(vampomi_ctx* c, const GramVec& gv, const MultiVec& mw) {
+    constexpr int C = GRAM_C;
+    const size_t smem = (size_t)GRAM_R * C * GRAM_ROWS * sizeof(double);
+    const auto kern = k_gram_wsx<K, CS>;
+    const size_t tr = (c->ld + CS - 1) / CS;
+    const int tile_rows = (int)((tr + 15) / 16 * 16);
+    CUtensorMap tm;
+    VO_CHECK(gram_tensor_map(c, tile_rows, C, &tm));
+    if (tile_rows > GRAM_ROWS) { set_error("gram: N=%d needs more than %d rows per CTA at cluster size %d", c->N, GRAM_ROWS, CS); return VAMPOMI_ERR_ARG; }
+    cudaLaunchConfig_t cfg = {};
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = CS; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+    cfg.blockDim = dim3(GRAM_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = c->stream; cfg.attrs = attr; cfg.numAttrs = 1;
+    // co-resident clusters of this (cluster size, systems) on this device: queried once per context
+    int& ncl = c->gram_clusters[CS][K - 1];
+    if (ncl <= 0) {
+        VO_CUDA(cudaFuncSetAttribute((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (CS > 8) VO_CUDA(cudaFuncSetAttribute((const void*)kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));   // 16 CTAs: one cluster per GPC
+        cfg.gridDim = dim3(CS, c->num_sms);
+        int n = 0;
+        if (cudaOccupancyMaxActiveClusters(&n, (const void*)kern, &cfg) != cudaSuccess || n < 1) { cudaGetLastError(); n = c->num_sms / CS; }
+        ncl = n < 1 ? 1 : n;
     }
-    set_error("gram: unknown shape %d", shape);
-    return VAMPOMI_ERR_ARG;
+    long long nch = c->tune.gram_clusters > 0 ? c->tune.gram_clusters : ncl;
+    const long long cap = (c->M + C - 1) / C;
+    if (nch > cap) nch = cap;
+    int cols_per_chunk = (int)((c->M + nch - 1) / nch);
+    cols_per_chunk = (cols_per_chunk + C - 1) / C * C;
+    const int nchunks = (int)((c->M + cols_per_chunk - 1) / cols_per_chunk);
+    VO_CHECK(ensure_ax_partial(c, (size_t)K * nchunks * c->ld));
+    cfg.gridDim = dim3(CS, nchunks);
+    if (c->prof_pending.size() > 8192) VO_CHECK(prof_resolve(c));
+    int sp = prof_begin(c, 3, (double)c->M * c->N * (double)c->elem_bytes);
+    const double scale = 1.0 / sqrt((double)c->N);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, (const double*)c->A, c->ld, (const double*)c->mave, (const double*)c->msig, gv, tile_rows,
+                                       cols_per_chunk, c->M, scale, c->ax_partial, nchunks, tm);
+    prof_end(c, sp);
+    if (e != cudaSuccess) { set_error("gram kernel launch failed: %s", cudaGetErrorString(e)); cudaGetLastError(); return VAMPOMI_ERR_CUDA; }
+    c->counters[0] += 1; c->counters[1]++; c->counters[2] += (long long)c->M * c->N * c->elem_bytes;
+    return launch_ax_reduce_multi(c, nchunks, mw);
 }
 
-template <int K>
-int gram_cluster(vampomi_ctx* c, const GramVec& gv, const MultiVec& mw) {
-    const int shape = c->tune.gram_shape;
-    int cs = c->tune.gram_cluster;
-    if (shape == 18) {
-        // the default shape runs on ANY cluster size up to 16 — the smallest that holds a column, so that a CTA's row tile (and with it
-        // the bytes a step moves per exchange) is as full as it can be: N = 12 000 on 5 CTAs x 2 400 rows instead of 8 x 1 500
-        // (tools/gram_large_n.py: a step costs ~1100 cycles whatever it carries)
-        if (cs == 0) cs = (int)((c->ld + gram_rows_of_shape(shape) - 1) / gram_rows_of_shape(shape));
-        switch (cs) {
-#define VAMPOMI_GRAM_CS(n) case n: return gram_launch_wsx<K, 8, 5, 2, n, 3, 0, 1>(c, gv, mw, shape);
-            VAMPOMI_GRAM_CS(1) VAMPOMI_GRAM_CS(2) VAMPOMI_GRAM_CS(3) VAMPOMI_GRAM_CS(4) VAMPOMI_GRAM_CS(5) VAMPOMI_GRAM_CS(6) VAMPOMI_GRAM_CS(7) VAMPOMI_GRAM_CS(8)
-            VAMPOMI_GRAM_CS(9) VAMPOMI_GRAM_CS(10) VAMPOMI_GRAM_CS(11) VAMPOMI_GRAM_CS(12) VAMPOMI_GRAM_CS(13) VAMPOMI_GRAM_CS(14) VAMPOMI_GRAM_CS(15) VAMPOMI_GRAM_CS(16)
-#undef VAMPOMI_GRAM_CS
-            default: set_error("gram: cluster size must be 1 ... 16"); return VAMPOMI_ERR_ARG;
-        }
-    }
-    if (cs == 0) { cs = 1; while (cs < gram_max_cluster_of_shape(shape) && (c->ld + cs - 1) / cs > (size_t)gram_rows_of_shape(shape)) cs *= 2; }
-    if (cs == 16) {
-        if (shape == 8) return gram_launch_ws<K, 10, 2, 4, 4, 16, 0>(c, gv, mw, shape);
-        if (shape == 11) return gram_launch_wsx<K, 10, 4, 2, 16, 2>(c, gv, mw, shape);     // 20 480 < N <= 40 960
-        if (shape == 12) return gram_launch_wsx<K, 8, 5, 2, 16, 3>(c, gv, mw, shape);
-        if (shape == 16) return gram_launch_wsx<K, 10, 4, 2, 16, 2, 0, 1>(c, gv, mw, shape);
-        set_error("gram: 16 CTAs per cluster only with shapes 8, 11, 12, 16 and 18");
-        return VAMPOMI_ERR_ARG;
-    }
-    switch (cs) {
-        case 1: return gram_shape<K, 1>(c, gv, mw, shape);
-        case 2: return gram_shape<K, 2>(c, gv, mw, shape);
-        case 4: return gram_shape<K, 4>(c, gv, mw, shape);
-        case 8: return gram_shape<K, 8>(c, gv, mw, shape);
-        default: set_error("gram: cluster size must be 1, 2, 4 or 8 for this shape"); return VAMPOMI_ERR_ARG;
-    }
-}
-
-}  // namespace
-
-// The instantiations for one system (K = 1) and for two (K = 2) compile independently: the Makefile builds this file twice, with
-// -DVAMPOMI_GRAM_K=1 (gram_run_k1 only) and -DVAMPOMI_GRAM_K=2 (everything else), to halve the build's longest step; without the
-// macro one translation unit holds both.
-#ifndef VAMPOMI_GRAM_K
-#define VAMPOMI_GRAM_K 0
-#endif
-
-namespace {
+// The cluster size is the smallest that holds a column (knob gram_cluster overrides it), so that a CTA's row tile — and with it the
+// bytes a step moves per exchange — is as full as it can be: N = 12 000 on 5 CTAs x 2 400 rows instead of 8 x 1 500 (a step
+// costs about the same number of cycles whatever it carries).
 template <int K>
 int gram_run(vampomi_ctx* c, const MultiVec& mq, double* const* w_out) {
     GramVec gv{};
@@ -1495,27 +483,27 @@ int gram_run(vampomi_ctx* c, const MultiVec& mq, double* const* w_out) {
         gv.q[k] = mq.in[k]; gv.t[k] = mq.out[k]; gv.done[k] = mq.done[k];
         mw.in[k] = nullptr; mw.out[k] = w_out[k]; mw.done[k] = mq.done[k];
     }
-    return gram_cluster<K>(c, gv, mw);
+    int cs = c->tune.gram_cluster;
+    if (cs == 0) cs = (int)((c->ld + GRAM_ROWS - 1) / GRAM_ROWS);
+    switch (cs) {
+#define VAMPOMI_GRAM_CS(n) case n: return gram_launch<K, n>(c, gv, mw);
+        VAMPOMI_GRAM_CS(1) VAMPOMI_GRAM_CS(2) VAMPOMI_GRAM_CS(3) VAMPOMI_GRAM_CS(4) VAMPOMI_GRAM_CS(5) VAMPOMI_GRAM_CS(6) VAMPOMI_GRAM_CS(7) VAMPOMI_GRAM_CS(8)
+        VAMPOMI_GRAM_CS(9) VAMPOMI_GRAM_CS(10) VAMPOMI_GRAM_CS(11) VAMPOMI_GRAM_CS(12) VAMPOMI_GRAM_CS(13) VAMPOMI_GRAM_CS(14) VAMPOMI_GRAM_CS(15) VAMPOMI_GRAM_CS(16)
+#undef VAMPOMI_GRAM_CS
+        default: set_error("gram: cluster size must be 1 ... 16"); return VAMPOMI_ERR_ARG;
+    }
 }
+
 }  // namespace
 
-int gram_run_k1(vampomi_ctx* c, const MultiVec& mq, double* const* w_out);
-#if VAMPOMI_GRAM_K != 2
-int gram_run_k1(vampomi_ctx* c, const MultiVec& mq, double* const* w_out) { return gram_run<1>(c, mq, w_out); }
-#endif
-
-#if VAMPOMI_GRAM_K != 1
-bool gram_supported(const vampomi_ctx* c) {
-    return c->storage == 0 && c->ld <= (size_t)gram_max_cluster_of_shape(c->tune.gram_shape) * gram_rows_of_shape(c->tune.gram_shape);
-}
+bool gram_supported(const vampomi_ctx* c) { return c->storage == 0 && c->ld <= (size_t)16 * GRAM_ROWS; }
 
 // t_k = A^T q_k (M-vectors), w_k = A t_k (N-vectors, summed over the GPUs, / sqrt(N)) for K <= 2 systems in ONE pass.
 // mq: in = q_k (N-vectors), out = t_k (M-vectors); w_out: the N-vectors that receive w_k. done flags from mq.
 int launch_gram(vampomi_ctx* c, const MultiVec& mq, double* const* w_out) {
     if (mq.K < 1 || mq.K > 2) { set_error("gram: 1 or 2 systems"); return VAMPOMI_ERR_ARG; }
     if (!gram_supported(c)) { set_error("gram: needs FP64 storage and N <= 40960"); return VAMPOMI_ERR_ARG; }
-    return mq.K == 1 ? gram_run_k1(c, mq, w_out) : gram_run<2>(c, mq, w_out);
+    return mq.K == 1 ? gram_run<1>(c, mq, w_out) : gram_run<2>(c, mq, w_out);
 }
-#endif
 
 }  // namespace vampomi
