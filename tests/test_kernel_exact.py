@@ -138,6 +138,12 @@ def test_stats_exact(N, M, storage, alpha):
         sh.upload(A)
         sh.compute_stats(alpha)
         mave, msig = sh.stats()
+    assert_stats_exact(held, mave, msig, alpha)
+
+
+def assert_stats_exact(held, mave, msig, alpha):
+    """mave / msig of the columns of `held` (as held on the device) against their exact values."""
+    N = held.shape[1]
     const = constant(held)
     # a constant column: its value and msig = 1, bit for bit (src/data.cpp:275-276 intends sumsqr == 0 for it)
     assert np.array_equal(mave[const], held[const, 0]), (np.nonzero(const)[0], mave[const] - held[const, 0])
@@ -278,12 +284,17 @@ def test_loo_sums_exact(N, M, storage):
     sh, held, mave, msig, rng = setup(N, M, storage, N * 13 + M)
     w = rng.standard_normal(N)
     sh.set(V_USER_N1, w)
-    got = sh.loo_sums(V_USER_N1)
+    assert_loo_sums_exact(sh.loo_sums(V_USER_N1), held, w)
+    sh.close()
+
+
+def assert_loo_sums_exact(got, held, w):
+    """sum x, sum x^2 and sum x w of the columns of `held` (rows of got) against their exact values."""
+    N = held.shape[1]
     h, wl = held.astype(LD), w.astype(LD)
     assert_within(got[:, 0], h.sum(axis=1), np.abs(h).sum(axis=1), N, "sum x")
     assert_within(got[:, 1], (h * h).sum(axis=1), (h * h).sum(axis=1), N, "sum x^2")
     assert_within(got[:, 2], (h * wl).sum(axis=1), np.abs(h * wl).sum(axis=1), N, "sum x w")
-    sh.close()
 
 
 @pytest.mark.parametrize("N,M", [(75777, 1), (2, 75776), (33, 1031)])

@@ -371,10 +371,16 @@ def test_cg_steps_exact(onepass):
     second solve is the state the first one returns). Iteration 2 uses the other parity slot of <r,z>."""
     N, M = 333, 517
     sh, A, rng = make_block(N, M, 31)
+    assert_cg_steps_exact(sh, onepass, rng.standard_normal(M), rng.standard_normal(M), 2.3, 0.7)
+    sh.close()
+
+
+def assert_cg_steps_exact(sh, onepass, v, v2, tau, gam2):
+    """Iterations 1 and 2 of cg_solve (right-hand side v) and of cg_solve_pair (v, v2) on the shard's block, each checked by
+    cg_step_check against the state before it."""
+    N, M = sh.N, sh.M
     sh.set_tuning("cg_onepass", onepass)
-    tau, gam2 = 2.3, 0.7
     diag = tau * (N - 1) / N + gam2
-    v, v2 = rng.standard_normal(M), rng.standard_normal(M)
     sh.set(V_V, v)
     sh.set(V_USER_M1, v2)
     init = dict(r=v, z=v / diag, p=v / diag, mu=np.zeros(M))
@@ -392,7 +398,6 @@ def test_cg_steps_exact(onepass):
             assert res[s][0] == k
             pair[s].append(snapshot(sh, s, vec, res[s][2]))
             cg_step_check(pair[s][k - 1], pair[s][k], rhs, tau, gam2, diag, M, f"cg_solve_pair system {s} onepass={onepass} iteration {k}")
-    sh.close()
 
 
 # ---- a long one-pass solve -------------------------------------------------------------------------------------------------
