@@ -17,7 +17,8 @@
 // A CTA is three warpgroups (THREADS = 384): two of compute warps (NCW = 8) and one SERVICE warpgroup — the communication warp,
 // the producer warp and two warps that only hand their registers over. Registers are allotted at launch as if every warp needed
 // the same (168 per thread); `setmaxnreg` then moves them: the service warpgroup drops to 96, the compute warpgroups rise to 200,
-// which their 5 row pairs of q, w and two steps of columns need. Eight compute warps put two on every scheduler.
+// which their 5 row pairs of q, w and two steps of columns need, plus the first PF row pairs of the next step (loaded ahead,
+// below). Eight compute warps put two on every scheduler.
 //
 // The columns arrive through a RING of R = 4 stages in shared memory. Each stage holds one step: ONE cp.async.bulk.tensor.3d
 // (SASS UTMALDG) per step brings both column pieces of the CTA's row tile (box 16 x tile/16 x C of the {16, ld/16, M} view of
@@ -28,12 +29,15 @@
 //
 // Step s, u = s % 4 (ring stage, exchange slot and barrier; the step loops are unrolled by four, so u is a compile-time offset
 // from one shared-window base register and the barrier parity is one bit flipped per trip):
-//   compute warp:        wait ringbar[u] -> LDS its row pairs, centre them, dot with q -> add the lane quadruples {l, l^8, l^16,
-//                        l^24} (two shuffle levels) -> red[u & 1], arrive on redbar[u];
+//   compute warp:        LDS the rest of its row pairs of stage u, centre them, dot with q -> add the lane quadruples {l, l^8,
+//                        l^16, l^24} (two shuffle levels) -> red[u & 1], arrive on redbar[u];
+//                        wait ringbar[(s+1) & 3] -> LDS the column means and the first PF row pairs of step s + 1 (LOADED AHEAD:
+//                        they arrive while the axpy below runs, so the next dot starts on data in registers);
 //                        wait wready[(s-1) & 3] -> read the weights -> axpy of step s - 1 on the registers that still hold its
 //                        centred columns (the axpy is DEFERRED by one step: a compute warp never waits for the cluster round
 //                        trip of the step it just dotted, only for the one before it)
-//   producer warp:       wait redbar[u] (every compute warp has read stage u) -> refill stage u with step s + 4
+//   producer warp:       wait redbar[u] (every compute warp has read stage u: the arrival follows the dot, which consumed the
+//                        loads of step s made one phase earlier as well as its own) -> refill stage u with step s + 4
 //   communication warp:  wait redbar[u] -> add the NCW warp sums (fixed tree) and the three shuffle levels left -> st.async the
 //                        CTA's partial sums to every CTA of the cluster (slot u) -> wait full[u] -> add the CS ranks' partial
 //                        sums by a fixed tree -> t_j (cluster rank 0 stores it) and the weight msig_j * t_j -> wbuf[u], arrive
@@ -68,6 +72,7 @@ constexpr int GRAM_NCW = 8;                                      // compute warp
 constexpr int GRAM_RP = 5;                                       // 16-byte row pairs per compute thread
 constexpr int GRAM_C = 2;                                        // columns per step
 constexpr int GRAM_R = 4;                                        // ring stages
+constexpr int GRAM_PF = 4;                                       // row pairs of the next step loaded during the axpy
 constexpr int GRAM_THREADS = (GRAM_NCW + 4) * 32;                // + the service warpgroup: 384
 constexpr int GRAM_ROWS = GRAM_NCW * 32 * GRAM_RP * 2;           // rows per CTA: 2 560
 
@@ -167,7 +172,8 @@ __global__ void __launch_bounds__(GRAM_THREADS, 1) k_gram_wsx(const double* __re
                                                              const double* __restrict__ msig, GramVec gv, int tile_rows, int cols_per_chunk,
                                                              long long M, double scale, double* __restrict__ partial, int nchunks,
                                                              const __grid_constant__ CUtensorMap tmap) {
-    constexpr int NCW = GRAM_NCW, RP = GRAM_RP, C = GRAM_C, R = GRAM_R;
+    constexpr int NCW = GRAM_NCW, RP = GRAM_RP, C = GRAM_C, R = GRAM_R, PF = GRAM_PF;
+    static_assert(PF <= C * RP, "at most one step ahead");
     constexpr int CK = C * K, LPV = 32 / CK, CT = NCW * 32, PIECE = CT * RP * 2;
     static_assert(C == 2 && (K == 1 || K == 2), "two columns per step: their means are one 16-byte load, their sums one or two value pairs");
     static_assert(CS <= 2 * LPV, "after the butterfly the LPV lanes that hold value ck send it to the CS ranks, at most two each");
@@ -326,21 +332,30 @@ __global__ void __launch_bounds__(GRAM_THREADS, 1) k_gram_wsx(const double* __re
         const uint32_t rows_u = opaque_u32(ring_u + (uint32_t)tid * 16u);             // this thread's first row pair inside a ring stage
         const uint32_t col_stride = (uint32_t)tile_rows * 8u;                         // bytes between the column pieces of a stage
 
-        auto dot_step = [&](const int u, const uint32_t par, const int s) {   // u = s % 4: ring stage, barrier; u & 1: register buffer, red slot
+        // The registers left beside q, w and two steps of columns hold PF row pairs: the next step's first ones and its column
+        // means are loaded while the axpy of the step before runs (a full step ahead would need ~240 registers)
+        double2 nx[PF], nm;
+        auto load_ahead = [&](const int u, const uint32_t par) {   // u: ring stage of the step, par: its barrier parity
+            mbar_spin_cta_u(cb + RINGBAR_O + 8 * u, par);
+            nm = lds_f64x2(cb + MST_O + (uint32_t)(u * C * 8));
+#pragma unroll
+            for (int p = 0; p < PF; p++)
+                nx[p] = lds_f64x2(rows_u + (uint32_t)((u * C * PIECE + (p % RP) * CT * 2) * 8) + (uint32_t)(p / RP) * col_stride);
+        };
+        auto dot_step = [&](const int u) {                       // u = s % 4: ring stage, barrier; u & 1: register buffer, red slot
             double pd[C][K][2];
 #pragma unroll
             for (int cc = 0; cc < C; cc++)
 #pragma unroll
                 for (int k = 0; k < K; k++) pd[cc][k][0] = pd[cc][k][1] = 0.0;
-            mbar_spin_cta_u(cb + RINGBAR_O + 8 * u, par);
-            const double2 mm = lds_f64x2(cb + MST_O + (uint32_t)(u * C * 8));
-            const double m[2] = {mm.x, mm.y};
+            const double m[2] = {nm.x, nm.y};
 #pragma unroll
             for (int cc = 0; cc < C; cc++)
 #pragma unroll
                 for (int i = 0; i < RP; i++) {
                     // rows beyond the tile read zeros or the next column's first rows: they only meet q = 0 and unsaved sums
-                    const double2 v = lds_f64x2(rows_u + (uint32_t)((u * C * PIECE + i * CT * 2) * 8) + (uint32_t)cc * col_stride);
+                    const double2 v = cc * RP + i < PF ? nx[cc * RP + i]
+                                                       : lds_f64x2(rows_u + (uint32_t)((u * C * PIECE + i * CT * 2) * 8) + (uint32_t)cc * col_stride);
                     const double d0 = v.x - m[cc], d1 = v.y - m[cc];            // meth[i] - mu, src/data.cpp:304 and :360
                     a[u & 1][cc][i][0] = d0; a[u & 1][cc][i][1] = d1;           // kept centred for the deferred axpy
 #pragma unroll
@@ -377,11 +392,13 @@ __global__ void __launch_bounds__(GRAM_THREADS, 1) k_gram_wsx(const double* __re
                     }
         };
         uint32_t ph = 0;
+        if (nsteps > 0) load_ahead(0, 0);
         for (int s0 = 0; s0 <= nsteps; s0 += 4, ph ^= 1u) {
 #pragma unroll
             for (int u = 0; u < 4; u++) {
                 const int s = s0 + u;
-                if (s < nsteps) dot_step(u, ph, s);
+                if (s < nsteps) dot_step(u);
+                if (s + 1 < nsteps) load_ahead((u + 1) & 3, u == 3 ? ph ^ 1u : ph);                    // step s + 1
                 if (s >= 1 && s <= nsteps) axpy_step((u + 3) & 3, u == 0 ? ph ^ 1u : ph, (u + 1) & 1);   // step s - 1
             }
         }
